@@ -2,6 +2,7 @@
 
     python bench.py [--gpus N --steps K --warmup W] [--impl reference|reference-cuda]
                     [--config cfg2|cfg1|cfg3|cfg4s|cfg5] [--beta B] [--precision auto|f32|f16|f16_split]
+                    [--dump-outputs DIR]
 
 A "step" is one `fit(V, beta, tol=-inf, max_iter=ITERS)` pass (the reference's own benchmark protocol,
 examples/benchmarks/benchmark.ipynb cell 4: loss evaluations every 10 iterations included) on one
@@ -178,6 +179,26 @@ class ClockSampler:
         wtop = watts[len(watts) // 2:] if watts else []     # board power under load (DESIGN.md 4.1: the cfg2 line sits at the cap)
         return {"sm_mhz": med, "sm_max_mhz": smax, "reasons": sorted(reasons), "samples": len(sm), "window": self.window,
                 "board_power_w": wtop[len(wtop) // 2] if wtop else None}
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write what the timed path returned as <out_dir>/<name>.npy in float32, so that two builds can be compared output
+    for output.  Past DUMP_BYTES in all, the largest array keeps a fixed, seeded sample of its rows (sorted)."""
+    import numpy as np
+    host = {k: v.detach().float().cpu() for k, v in arrays.items()}
+    total = sum(t.numel() * 4 for t in host.values())
+    if total > DUMP_BYTES:
+        k = max(host, key=lambda n: host[n].numel())
+        t = host[k]
+        rows = (DUMP_BYTES - (total - t.numel() * 4)) // (t[0].numel() * 4)
+        idx = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:rows].sort().values
+        host[k] = t[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    for k, t in host.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), t.numpy())
 
 
 def dist_setup(n_gpus):
@@ -472,6 +493,8 @@ def main():
     ap.add_argument("--no-gpu-reference", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip north_star_cfg4 / sharded_check")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write W and H of the last timed step (rank 0's shard) to DIR/W.npy, DIR/H.npy (float32, <= 64 MB)")
     a = ap.parse_args()
     kind, shape, beta, desc = CONFIGS[a.config]
     if beta is None:
@@ -535,6 +558,8 @@ def main():
     clocks = sampler.stop() if sampler else None
     precision = model.last_fit_precision
     value = a.iters * a.steps * world / (ms * 1e-3)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"W": model.W.data, "H": model.H.data})
 
     # ---------------- end to end through the public API with host buffers ------------------------------
     e2e = None

@@ -8,7 +8,9 @@ the reference is importable from /root/reference (read-only) or baseline/_ref:
 
 The GPU box has no reference; the fixtures written here are what travels.  Inputs are generated
 from fixed torch CPU seeds (SURVEY 8d): V = rand(N,C) rounded to bf16-representable values, so the
-fp32 reference and the 16-bit-operand engine consume bit-identical data; W0/H0 = |randn|.
+fp32 reference and the 16-bit-operand engine consume bit-identical data; W0/H0 = |randn|.  The fixtures store
+the reference's outputs and, in place of the inputs, the recipe of oracle/golden_inputs.py that regenerates them
+with their sha256 (every file stays under 1 MB).
 """
 import argparse
 import math
@@ -18,6 +20,8 @@ import time
 
 import numpy as np
 import torch
+
+import golden_inputs as gi
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 for cand in (os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
@@ -102,7 +106,14 @@ def small_cases():
     return cases
 
 
-def save_cases(cases, fname):
+def factor_args(V, W0, H0, **kw):
+    """Arguments of the `factors` recipe (oracle/golden_inputs.py) that regenerates these make_inputs tensors."""
+    return dict(v_shape=list(V.shape), w_shape=list(W0.shape), h_shape=list(H0.shape), **kw)
+
+
+def save_cases(cases, fname, inputs=None):
+    """`inputs(case) -> (recipe, args)` names the recipe of the case's V, W0, H0; by default make_inputs' own, with the
+    floor it applies for beta <= 0."""
     flat = {}
     for name, c in cases.items():
         for k, v in c.items():
@@ -115,6 +126,9 @@ def save_cases(cases, fname):
             else:
                 v = np.array(v, dtype=np.float64)
             flat[f"{name}/{k}"] = v
+        recipe, args = inputs(c) if inputs else (
+            "factors", factor_args(c["V"], c["W0"], c["H0"], floor=2 ** -7 if c["beta"] <= 0 else 0.0))
+        gi.pack(flat, name, recipe, **args)
     os.makedirs(GOLD, exist_ok=True)
     np.savez_compressed(os.path.join(GOLD, fname), **flat)
     print(f"wrote {fname}: {len(cases)} cases, {os.path.getsize(os.path.join(GOLD, fname)) / 1e6:.2f} MB")
@@ -149,7 +163,7 @@ def cfg2_case(iters=200):
 # ---------------------------------------------------------------------------------------------------------
 def _store(flat, name, V, W0, H0, W, H, n_iter, losses, meta, w_step=1, h_step=1):
     flat[f"{name}/W_sub"] = W[::w_step].numpy()
-    flat[f"{name}/H_sub"] = (H[::h_step] if H.dim() == 2 else H).numpy()
+    flat[f"{name}/H_sub"] = (H[::h_step] if H.dim() == 2 else H[..., ::h_step]).contiguous().numpy()
     flat[f"{name}/w_step"] = np.array(w_step); flat[f"{name}/h_step"] = np.array(h_step)
     flat[f"{name}/n_iter"] = np.array(n_iter)
     flat[f"{name}/losses"] = np.array(losses, dtype=np.float64)
@@ -178,7 +192,7 @@ def round2_cases():
     V, W0, H0 = make_inputs((B, C, L), (C, R, T), (B, R, L - T + 1))
     W, H, n_iter, losses = run_reference(ref_nmf.NMFD, V, W0, H0, 1, float("-inf"), 20, 0, 0)
     _store(flat, "nmfd_cfg3", V, W0, H0, W, H, n_iter, losses,
-           dict(B=B, C=C, L=L, R=R, T=T, beta=1, max_iter=20), w_step=8)
+           dict(B=B, C=C, L=L, R=R, T=T, beta=1, max_iter=20), w_step=64, h_step=8)
     print(f"nmfd_cfg3 {time.time() - t0:.1f}s", flush=True)
     # --- NMFD ragged: T = 37 crosses the 32-wide shift chunk, C = 130 crosses the 128-row tile, batch 2 ---
     B, C, L, R, T = 2, 130, 700, 5, 37
@@ -186,13 +200,13 @@ def round2_cases():
         V, W0, H0 = make_inputs((B, C, L), (C, R, T), (B, R, L - T + 1))
         W, H, n_iter, losses = run_reference(ref_nmf.NMFD, V, W0, H0, beta, float("-inf"), 20, 0, 0)
         _store(flat, f"nmfd_ragged_b{beta}", V, W0, H0, W, H, n_iter, losses,
-               dict(B=B, C=C, L=L, R=R, T=T, beta=beta, max_iter=20))
+               dict(B=B, C=C, L=L, R=R, T=T, beta=beta, max_iter=20), w_step=2)
     print(f"nmfd_ragged {time.time() - t0:.1f}s", flush=True)
     # --- cfg4-shaped: R = 128 (the 128-column operand kernels), KL, 100 iterations ---
     N, C, R = 8192, 2048, 128
     V, W0, H0 = make_inputs((N, C), (C, R), (N, R))
     W, H, n_iter, losses = run_reference(ref_nmf.NMF, V, W0, H0, 1, float("-inf"), 100, 0, 0)
-    _store(flat, "nmf_r128_kl", V, W0, H0, W, H, n_iter, losses, dict(N=N, C=C, R=R, beta=1, max_iter=100), h_step=8)
+    _store(flat, "nmf_r128_kl", V, W0, H0, W, H, n_iter, losses, dict(N=N, C=C, R=R, beta=1, max_iter=100), w_step=8, h_step=64)
     print(f"nmf_r128 {time.time() - t0:.1f}s", flush=True)
     # --- cfg5-shaped: beta sweep at R = 64, 50 iterations ---
     N, C, R = 4096, 1024, 64
@@ -200,7 +214,7 @@ def round2_cases():
         V, W0, H0 = make_inputs((N, C), (C, R), (N, R), floor=2 ** -7 if beta <= 0 else 0.0)
         W, H, n_iter, losses = run_reference(ref_nmf.NMF, V, W0, H0, beta, float("-inf"), 50, 0, 0)
         _store(flat, f"nmf_sweep_b{beta}", V, W0, H0, W, H, n_iter, losses,
-               dict(N=N, C=C, R=R, beta=beta, max_iter=50, floor=2 ** -7 if beta <= 0 else 0.0), h_step=4)
+               dict(N=N, C=C, R=R, beta=beta, max_iter=50, floor=2 ** -7 if beta <= 0 else 0.0), w_step=16, h_step=64)
     print(f"sweep {time.time() - t0:.1f}s", flush=True)
     # --- heavy-tailed targets (lognormal, ~6 decades): KL and IS, 30 iterations ---
     N, C, R = 1024, 512, 32
@@ -210,7 +224,7 @@ def round2_cases():
         W0 = torch.randn(C, R).abs(); H0 = torch.randn(N, R).abs()
         W, H, n_iter, losses = run_reference(ref_nmf.NMF, V, W0, H0, beta, float("-inf"), 30, 0, 0)
         _store(flat, f"nmf_heavy_b{beta}", V, W0, H0, W, H, n_iter, losses,
-               dict(N=N, C=C, R=R, beta=beta, max_iter=30))
+               dict(N=N, C=C, R=R, beta=beta, max_iter=30), w_step=4, h_step=8)
     np.savez_compressed(os.path.join(GOLD, "reference_r2.npz"), **flat)
     print(f"wrote reference_r2.npz ({os.path.getsize(os.path.join(GOLD, 'reference_r2.npz')) / 1e6:.2f} MB) in {time.time() - t0:.1f}s")
 
@@ -246,6 +260,7 @@ def next_row_cases():
                 flat[f"{name}/{k}"] = v.numpy()
             for k, v in dict(beta=beta, l1=l1, l2=l2, ortho=ortho, steps=3).items():
                 flat[f"{name}/{k}"] = np.array(v, dtype=np.float64)
+            gi.pack(flat, name, "factors", **factor_args(V, W0, H0, offset=2 ** -7 if beta <= 0 else 0.0))
     # --- PLCA: small ragged case (Dirichlet priors, frozen Z) and a tensor-core-shaped case ---
     for name, (N, C, R, iters, kw, fitkw) in {
         "plca_small": (97, 83, 8, 30, {}, {}),
@@ -266,6 +281,7 @@ def next_row_cases():
         flat[f"{name}/trainable_Z"] = np.array(int(kw.get("trainable_Z", True)))
         for k in ("W_alpha", "H_alpha", "Z_alpha"):
             flat[f"{name}/{k}"] = np.array(float(fitkw.get(k, 1.0)))
+        gi.pack(flat, name, "factors", **factor_args(V, W0, H0, scale=3, z=True))
     np.savez_compressed(os.path.join(GOLD, "reference_next.npz"), **flat)
     print(f"wrote reference_next.npz ({os.path.getsize(os.path.join(GOLD, 'reference_next.npz')) / 1e6:.2f} MB)")
 
@@ -310,6 +326,7 @@ def plca_cases():
             flat[f"{name}/{k}"] = np.array(int(kw.get(k, True)))
         for k in ("W_alpha", "H_alpha", "Z_alpha"):
             flat[f"{name}/{k}"] = np.array(float(fitkw.get(k, 1.0)))
+        gi.pack(flat, name, "factors", **factor_args(V, W0, H0, scale=3, z=True))
         print(name, "n_iter", n_iter)
     # --- BetaMu over the convolutive modules (trainer.py:36-121 with NMFD / NMF2D / NMF3D as the single leaf) ---
     import torchnmf.trainer as ref_trainer
@@ -337,6 +354,7 @@ def plca_cases():
                     flat[f"{name}/{k}"] = v.numpy()
                 for k, v in dict(beta=beta, l1=l1, l2=l2, ortho=ortho, steps=3, nd=len(K)).items():
                     flat[f"{name}/{k}"] = np.array(v, dtype=np.float64)
+                gi.pack(flat, name, "factors", **factor_args(V, W0, H0, offset=2 ** -7 if beta <= 0 else 0.0))
     np.savez_compressed(os.path.join(GOLD, "reference_plca.npz"), **flat)
     print(f"wrote reference_plca.npz ({os.path.getsize(os.path.join(GOLD, 'reference_plca.npz')) / 1e6:.2f} MB)")
 
@@ -364,7 +382,8 @@ def sparse_cases():
         W, H, n_iter, losses = run_reference(ref_nmf.NMF, Vs, W0, H0, beta, 1e-3, 100, 0, 0)
         cases[f"sparse_b{beta}_stoprule"] = dict(kind="nmf", V=D, W0=W0, H0=H0, W=W, H=H, n_iter=n_iter, losses=losses,
                                                  beta=beta, tol=1e-3, max_iter=100, alpha=0, l1_ratio=0)
-    save_cases(cases, "reference_sparse.npz")
+    save_cases(cases, "reference_sparse.npz", inputs=lambda c: (
+        "thresholded", dict(shape=[N, C], rank=R, keep_above=0.93, seeds=[0, 1], empty_row=17, empty_col=5)))
 
 
 def nd_cases():
@@ -433,6 +452,7 @@ def hoyer_cases():
                 Y[sl] = ref_nmf._proj_func(X[sl].clone(), float(k1[j]), float(k2[j]))
             put(f"{name}_{form}", dict(X=X, Y=Y, k1=torch.tensor(k1, dtype=torch.float64),
                                        k2=torch.tensor(k2, dtype=torch.float64)), dict(dim=dim))
+            gi.pack(flat, f"{name}_{form}", "proj_slices", shape=list(shape), negative_row=name == "proj_dim0")
 
     # --- sparse_fit (nmf.py:411-599) ---
     def run_sfit(name, cls, vshape, wshape, hshape, beta, iters, sW, sH, **kw):
@@ -442,6 +462,7 @@ def hoyer_cases():
         put(name, dict(V=V, W0=W0, H0=H0, W=m.W, H=m.H),
             dict(beta=beta, iters=iters, n_iter=n_iter, sW=-1 if sW is None else sW, sH=-1 if sH is None else sH,
                  trainable_W=int(kw.get("trainable_W", True)), trainable_H=int(kw.get("trainable_H", True))))
+        gi.pack(flat, name, "factors", **factor_args(V, W0, H0, floor=2 ** -7 if beta <= 0 else 0.0))
 
     N, C, R = 97, 83, 8
     nmf = ref_nmf.NMF
@@ -472,6 +493,7 @@ def hoyer_cases():
         n_iter = m.sparse_fit(Vd.to_sparse(), 2, 8, False, sW, sH)
         put(name, dict(V=Vd, W0=W0, H0=H0, W=m.W, H=m.H),
             dict(beta=2, iters=8, n_iter=n_iter, sW=-1 if sW is None else sW, sH=-1 if sH is None else sH))
+        gi.pack(flat, name, "thresholded", shape=[200, 150], rank=8, keep_above=0.9, seeds=[5, 6], bf16=True)
 
     # --- trainer.SparsityProj (trainer.py:124-190): steps on one NMF module, closure = beta_div of its reconstruction ---
     # (short runs: once the loss flattens, `loss <= init_loss` is decided by rounding and the step sizes of two
@@ -492,6 +514,7 @@ def hoyer_cases():
         losses = [float(tr.step(closure)) for _ in range(steps)]
         put(name, dict(V=V, W0=W0, H0=H0, W=m.W, H=m.H, losses=torch.tensor(losses, dtype=torch.float64)),
             dict(beta=beta, sparsity=sp, steps=steps, lr0=lr0, lr=tr.param_groups[0]["lr"], on_W=int("W" in which), on_H=int("H" in which)))
+        gi.pack(flat, name, "factors", **factor_args(V, W0, H0, floor=0.0))
     np.savez_compressed(os.path.join(GOLD, "reference_hoyer.npz"), **flat)
     print(f"wrote reference_hoyer.npz ({os.path.getsize(os.path.join(GOLD, 'reference_hoyer.npz')) / 1e6:.2f} MB)")
 

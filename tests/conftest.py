@@ -13,14 +13,30 @@ for p in (ROOT, PKG):
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 
+from oracle import golden_inputs  # noqa: E402
+
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
 
 
+class Fixture(dict):
+    """{"<case>/<field>": array} of one fixture file, keyed like np.load's result (`files` included)."""
+
+    @property
+    def files(self):
+        return list(self)
+
+
+def load_npz(fname):
+    """A fixture written by oracle/make_golden.py, with the inputs it stores as seeded recipes regenerated and checked."""
+    with np.load(os.path.join(GOLDEN, fname), allow_pickle=False) as z:
+        return Fixture(golden_inputs.unpack({k: z[k] for k in z.files}))
+
+
 def load_golden(fname="reference_small.npz"):
     """Return {case_name: {field: value}} from a fixture written by oracle/make_golden.py."""
-    z = np.load(os.path.join(GOLDEN, fname), allow_pickle=False)
+    z = load_npz(fname)
     cases = {}
     for key in z.files:
         name, field = key.split("/", 1)

@@ -2,8 +2,8 @@
 (tests/golden/reference_r2.npz, written by `python oracle/make_golden.py --r2` from the real torchnmf 0.3.5).
 
 Inputs are regenerated from the fixture's seeds and verified against its float64 checksums; only subsampled
-factors are stored.  Tolerance everywhere: the north-star's rtol 1e-3 with atol = 1e-5 * max|factor| for the
-near-zero entries multiplicative updates produce.
+factors are stored (rows at a stride, the H of NMFD along its last axis).  Tolerance everywhere: the north-star's
+rtol 1e-3 with atol = 1e-5 * max|factor| for the near-zero entries multiplicative updates produce.
 """
 import math
 import os
@@ -48,7 +48,7 @@ def _compare(c, m, label, rtol=RTOL):
     ws, hs = int(c["w_step"]), int(c["h_step"])
     W = m.W.data.cpu()[::ws]
     H = m.H.data.cpu()
-    H = H[::hs] if H.dim() == 2 else H
+    H = H[::hs] if H.dim() == 2 else H[..., ::hs]
     worst = 0.0
     for got, want, mx, nm in ((W, torch.from_numpy(c["W_sub"]), float(c["w_absmax"]), "W"),
                               (H, torch.from_numpy(c["H_sub"]), float(c["h_absmax"]), "H")):

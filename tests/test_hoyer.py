@@ -6,13 +6,11 @@ CPU tests: the oracle restatement (oracle/hoyer_oracle.py) against the reference
 and `SparsityProj` with the oracle standing in for the library.  GPU tests: `nmfb200_hoyer_project`, `sparse_fit` and
 `SparsityProj` through the C ABI against the same fixtures (rtol 1e-3, atol 1e-5 * max: the north-star tolerance).
 """
-import os
-
 import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN
+from conftest import load_npz
 from oracle import hoyer_oracle as hoy
 from oracle import mu_oracle as orc
 from oracle_engine import OracleNmfEngine, OracleNmfdEngine
@@ -22,7 +20,7 @@ from torchnmf_b200 import engine as _engine
 from torchnmf_b200 import trainer as _trainer
 from torchnmf_b200.metrics import beta_div, sparseness
 
-Z = np.load(os.path.join(GOLDEN, "reference_hoyer.npz"), allow_pickle=False)
+Z = load_npz("reference_hoyer.npz")
 NAMES = sorted({k.split("/")[0] for k in Z.files})
 PROJ = [n for n in NAMES if n.startswith("proj_")]
 SFIT = [n for n in NAMES if n.startswith("sfit_")]

@@ -8,18 +8,16 @@ CPU tests: the closed-form oracle (oracle/plca_oracle.py) against those fixtures
 surface (constructors, shapes, normalisation, reconstruct).  GPU tests: `fit` through the C ABI
 (`nmfb200_nmf_raw_terms` / `nmfb200_nmfd_raw_terms`) against the same fixtures at rtol 1e-3.
 """
-import os
-
 import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN
+from conftest import load_npz
 from oracle import plca_oracle
 from torchnmf_b200 import PLCA, SIPLCA, SIPLCA2, SIPLCA3, NMFD, NMF2D, NMF3D, BetaMu
 
-ZN = np.load(os.path.join(GOLDEN, "reference_next.npz"), allow_pickle=False)
-ZP = np.load(os.path.join(GOLDEN, "reference_plca.npz"), allow_pickle=False)
+ZN = load_npz("reference_next.npz")
+ZP = load_npz("reference_plca.npz")
 CLS = {0: PLCA, 1: SIPLCA, 2: SIPLCA2, 3: SIPLCA3}
 
 

@@ -1,9 +1,10 @@
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "pytorch-nmf_b200"), os.path.join(ROOT, "tests")]
-import numpy as np, torch
+import torch
+from conftest import load_npz
 from torchnmf_b200 import PLCA
-Z = np.load(os.path.join(ROOT, "tests", "golden", "reference_next.npz"))
+Z = load_npz("reference_next.npz")
 def case(name): return {k.split("/", 1)[1]: Z[k] for k in Z.files if k.startswith(name + "/")}
 for name in ("plca_small", "plca_prior", "plca_frozenZ", "plca_tc"):
     c = case(name)
