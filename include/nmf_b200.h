@@ -98,8 +98,7 @@ int nmfb200_nmf_update_w(nmfb200_ctx* ctx, float* W, const float* H,
 int nmfb200_nmf_update_h(nmfb200_ctx* ctx, const float* W, float* H,
                          double beta, double gamma, double l1_reg, double l2_reg, void* stream);
 /* n_iter consecutive MU iterations with both factors trainable: exactly n_iter x (update_w; update_h), i.e.
- * nmf.py:366-391 repeated, in one host call.  With NMFB200_GRAPH=1 the tensor-core path captures the iteration
- * into a CUDA graph and replays it (measured: no gain, the stream is not launch-bound); results are identical. */
+ * nmf.py:366-391 repeated, in one host call. */
 int nmfb200_nmf_iterate(nmfb200_ctx* ctx, float* W, float* H, double beta, double gamma, double l1_reg,
                         double l2_reg, int n_iter, void* stream);
 /* beta_div(H W^T, V, beta) (metrics.py:60-96) accumulated into the DEVICE double *loss_dev

@@ -18,10 +18,6 @@ NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr",
 ]
-if os.environ.get("NMFB200_BUILD_TRACE"):       # tuning build (tools/tc_trace.py, tc_knock.py): separate library, loaded
-    NVCC_FLAGS += ["-DNMFB200_TRACE"]           # with NMFB200_LIB=<...>/lib/trace/libnmf_b200.so
-    LIBDIR = os.path.join(LIBDIR, "trace")
-    LIB = os.path.join(LIBDIR, "libnmf_b200.so")
 
 
 def _nvcc():

@@ -12,8 +12,7 @@ namespace nmfb200 {
 static thread_local std::string g_err;
 static std::atomic<int64_t> g_launches{0};
 void set_error(const std::string& msg) { g_err = msg; }
-void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
-int64_t launch_counter() { return g_launches.load(); }
+void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 }  // namespace nmfb200
 
 using namespace nmfb200;

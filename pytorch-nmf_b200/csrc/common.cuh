@@ -21,8 +21,7 @@ inline BetaMode beta_mode(double beta) {
 }
 
 void set_error(const std::string& msg);
-void count_launch(int n = 1);
-int64_t launch_counter();
+void count_launch();
 
 #define NMF_CUDA_CHECK(expr)                                                              \
   do {                                                                                    \
@@ -45,6 +44,18 @@ int64_t launch_counter();
 
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 static inline int64_t round_up(int64_t a, int64_t b) { return ceil_div(a, b) * b; }
+
+// The element step of the multiplicative update (nmf.py:78-92) once the numerator `num` and the denominator `pos` of
+// element `v` are formed: v ((relu(num) + eps) / (pos [+ l1] [+ l2 v]))^gamma.  Each ratio-stage kernel sums its own
+// partials and forms `pos` (relu(den) + eps, or the KL column sum); the tail is this one.
+__device__ __forceinline__ float mu_step(float v, float num, float pos, float l1, float l2, float gamma) {
+  const float neg = fmaxf(num, 0.f) + kEps;              // nmf.py:78
+  if (l1 > 0.f) pos += l1;                               // nmf.py:85-86
+  if (l2 > 0.f) pos = fmaf(l2, v, pos);                  // nmf.py:87-88
+  float mult = neg / pos;                                // nmf.py:89
+  if (gamma != 1.0f) mult = powf(mult, gamma);           // nmf.py:90-91
+  return v * mult;                                       // nmf.py:92
+}
 
 // ------------------------------------------------------------------------------------------
 // Launch wrappers implemented in the .cu files (all asynchronous on `st`, return 0 / error code)

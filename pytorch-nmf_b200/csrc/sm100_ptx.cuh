@@ -52,9 +52,8 @@ __device__ __forceinline__ bool mbar_test_wait(uint32_t bar, uint32_t parity) {
   return ok != 0;
 }
 // try_wait with a suspend-time hint: the hardware parks the thread until the phase completes or the hint expires instead of
-// returning after a few tens of cycles (CUTLASS passes the same 0x989680).  Staged for round 2 behind NMFB200_TC_PARK in
-// the tuning build: the unparked poll loops execute ~4 M try_wait per launch (ncu source page), a quarter of the SM's
-// issue slots and avoidable power on a power-capped part; one cross-box measurement showed no gain.
+// returning after a few tens of cycles (CUTLASS passes the same 0x989680).  Unparked poll loops executed ~4 M try_wait per
+// launch (ncu source page), a quarter of the SM's issue slots and avoidable power on a power-capped part.
 __device__ __forceinline__ bool mbar_try_wait_parked(uint32_t bar, uint32_t parity) {
   uint32_t ok;
   asm volatile(
@@ -66,9 +65,6 @@ __device__ __forceinline__ bool mbar_try_wait_parked(uint32_t bar, uint32_t pari
       : "memory");
   return ok != 0;
 }
-#ifdef NMFB200_TRACE
-static __device__ unsigned int g_tune_park;      // tuning build: non-zero = parked polls in mbar_wait_slow
-#endif
 // Bounded wait: on a protocol bug (no progress for ~1 s) the first waiter records (block, thread, barrier, parity)
 // in g_wait_abort and every wait in the grid then falls through, so the kernel terminates instead of hanging
 // the GPU box; the host checks the record after the launch (tc_nmf.cu: check_wait_abort).
@@ -81,15 +77,7 @@ static __device__ unsigned int g_wait_abort[8];      // one record per translati
 static __device__ __noinline__ void mbar_wait_slow(uint32_t bar, uint32_t parity) {
   uint32_t polls = 0;
   long long t0 = 0;
-#ifdef NMFB200_TRACE
-  const unsigned int mode = *reinterpret_cast<volatile unsigned int*>(&g_tune_park);
-  const bool park = mode != 2u;            // tuning build: NMFB200_TC_PARK=2 restores the plain poll loop
-#else
-  constexpr bool park = true;       // parked polls: +1 % sustained at cfg2 (power-capped part), nothing in a burst
-  constexpr unsigned int mode = 0u;
-#endif
-  while (!(park ? mbar_try_wait_parked(bar, parity) : mbar_try_wait(bar, parity))) {
-    if (mode >= 2u) __nanosleep(mode);          // tuning: back-off between polls (issue slots of the spinning warps)
+  while (!mbar_try_wait_parked(bar, parity)) {      // parked polls: +1 % sustained at cfg2 (power-capped part), nothing in a burst
     if ((++polls & 1023u) != 0u) continue;
     if (*reinterpret_cast<volatile unsigned int*>(&g_wait_abort[0]) != 0u) return;
     const long long now = clock64();
@@ -116,13 +104,6 @@ __device__ __forceinline__ void tma_load_2d(const CUtensorMap* m, uint32_t bar, 
       "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
       ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(x), "r"(y)
       : "memory");
-}
-
-// fire-and-forget prefetch of one box into L2 (no shared memory, no mbarrier)
-__device__ __forceinline__ void tma_prefetch_l2_2d(const CUtensorMap* m, int x, int y) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];"
-               ::"l"(reinterpret_cast<uint64_t>(m)), "r"(x), "r"(y)
-               : "memory");
 }
 
 // ---- tcgen05 ------------------------------------------------------------------------------------
@@ -236,18 +217,6 @@ __device__ __forceinline__ bool elect_one() {
 }
 
 // ---- small math helpers ----------------------------------------------------------------------------
-// Reciprocal on the FMA pipe (x > 0, normal): integer seed (<= 12 % off) + three Newton steps -> < 1e-7 relative.
-// Staged for round 2 (tuning build, knock bit 64): moves a quarter of the ratio stage's reciprocals off the XU pipe,
-// which needs 1024 of the ~1250 cycles a tile spends in the ratio stage (DESIGN.md 9).
-__device__ __forceinline__ float rcp_fma(float x) {
-  float r = __int_as_float(0x7EF311C7 - __float_as_int(x));
-  float e = fmaf(-x, r, 1.f);
-  r = fmaf(r, e, r);
-  e = fmaf(-x, r, 1.f);
-  r = fmaf(r, e, r);
-  e = fmaf(-x, r, 1.f);
-  return fmaf(r, e, r);
-}
 __device__ __forceinline__ float rcp_approx(float x) {
   float r;
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));

@@ -28,7 +28,6 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
-#include <vector>
 
 #include "sm100_ptx.cuh"
 
@@ -46,14 +45,12 @@ constexpr uint32_t kColS = 0;        // S/P stages: columns [TN i, TN i + TN); O
 //   NF / NG / NV  F blocks, G-tile ring, V-tile ring;  NS  S/P accumulator stages in TMEM (the S-MMA warp runs up to
 //   NS tiles ahead of the O-MMA warp)
 //   NRW   ratio warpgroups (each processes TN / NRW columns of every tile)
-//   NP    0: the ratio tile P is written over the S columns of its stage (the stage is free again when the O-MMA has
-//         consumed P).  > 0: P has NP buffers of TN / 2 columns of its own: an S stage is handed back as soon as the
-//         ratio warps have READ it, a P buffer when its O-MMA has completed -- two short rings instead of one long one.
+// The ratio tile P is written over the S columns of its stage; the stage is free again when the O-MMA has consumed P.
 constexpr unsigned kEpiPaceNs = 100;     // pause between the epilogue's row stores (see the epilogue warpgroup)
 
-template <int RP_, bool SPLIT_, int TN_, int NF_, int NG_, int NV_, int NS_, int NRW_ = 2, int NP_ = 0>
+template <int RP_, bool SPLIT_, int TN_, int NF_, int NG_, int NV_, int NS_, int NRW_ = 2>
 struct Cfg {
-  static constexpr int RP = RP_, TN = TN_, NF = NF_, NG = NG_, NV = NV_, NS = NS_, NRW = NRW_, NP = NP_;
+  static constexpr int RP = RP_, TN = TN_, NF = NF_, NG = NG_, NV = NV_, NS = NS_, NRW = NRW_;
   // 4 NRW ratio warps, then 4 epilogue warps, then 4 control warps (TMA V / MMA S / TMA F,G / MMA O)
   static constexpr int kThreads = 128 + 128 * NRW_ + 128;
   static constexpr bool SPLIT = SPLIT_;
@@ -73,26 +70,10 @@ struct TcKernelParams {
   int ef, eg;                 // which of exps[] belong to F and G
   double* loss_part;          // LOSS mode: [gridDim.x][2] = {sum v~ lg2(x), sum S~}
   const float* kappa;         // device scalar: centring constant of the ratio tile (typical P), 0 = off
-  int pf_dist;                // L2 prefetch distance of the V stream in tiles (0 = off)
-  long long* trace;           // tuning aid: per-tile event timestamps of CTA 0 ([tile][16]), or nullptr
-  int knock;                  // tuning build only (NMFB200_TC_KNOCK): bit mask of pipeline stages to skip
 };
 
-// Event timeline of CTA 0 (tools/tc_trace.py): compiled in only with -DNMFB200_TRACE (build.py: NMFB200_BUILD_TRACE=1);
-// the product build carries no trace code in the warp-specialised loops.
-#ifdef NMFB200_TRACE
-#define TC_TRACE(tile, k)                                                        \
-  do {                                                                         \
-    if (p.trace && blockIdx.x == 0 && (tile) < 256) p.trace[(tile) * 16 + (k)] = clock64(); \
-  } while (0)
-#define TC_KNOCK(bit) ((p.knock & (bit)) != 0)      // knock-out experiments (results invalid): which stage bounds the kernel?
-#else
-#define TC_TRACE(tile, k) do { } while (0)
-#define TC_KNOCK(bit) false
-#endif
-
 // shared memory: NF F blocks | NG G-tile ring | NV V-tile ring | mbarriers | tmem ptr | loss slots
-template <int KW, int TN, int NF, int NG, int NV, int NS, int NP = 0>
+template <int KW, int TN, int NF, int NG, int NV, int NS>
 struct SmemLayout {
   static constexpr int kFBytes = kTileM * KW * 2;
   static constexpr int kGBytes = TN * KW * 2;
@@ -101,8 +82,8 @@ struct SmemLayout {
   static constexpr int kG = kF + NF * kFBytes;
   static constexpr int kV = kG + NG * kGBytes;
   static constexpr int kBar = kV + NV * kVBytes;
-  static constexpr int kNumBars = 2 * NF + 2 * NG + 2 * NV + 2 * NS + 2 * (NP ? NP : NS) + 2;
-  static constexpr int kTmemPtr = kBar + 8 * kNumBars;
+  static constexpr int kNumBars = 2 * NF + 2 * NG + 2 * NV + 3 * NS + 2;
+  static constexpr int kTmemPtr = (kBar + 8 * kNumBars + 15) / 16 * 16;   // loss slots 16-byte aligned: paired doubles
   static constexpr int kLossSlots = kTmemPtr + 16;
   static constexpr int kTotal = kLossSlots + 16 * 16;
 };
@@ -136,16 +117,11 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
   constexpr bool EU = BM == kBmEU;
   // TMEM columns.  one-output: S/P stages [0, NS TN) | O [NS TN, NS TN + KW).
   //               two-output: S/Pn stages [0, 256) | Pp stages [256, 384) | O_num [384, 448) | O_den [448, 512)
-  constexpr int NP = C::NP;
-  constexpr bool PSEP = NP > 0;                   // P in buffers of its own (one-output update kernels only)
-  constexpr int NPB = PSEP ? NP : NS;             // P-full / P-empty barriers
   constexpr uint32_t kColPp = NS * TN;
-  constexpr uint32_t kColP = NS * TN;             // PSEP: P buffer b = columns [kColP + b TN/2, + TN/2)
-  constexpr uint32_t kColO = TWO ? 384 : (PSEP ? NS * TN + NP * (TN / 2) : NS * TN);
+  constexpr uint32_t kColO = TWO ? 384 : NS * TN;
   constexpr uint32_t kColO2 = 448;
-  using L = SmemLayout<KW, TN, NF, NG, NV, NS, NP>;
+  using L = SmemLayout<KW, TN, NF, NG, NV, NS>;
   static_assert(TWO || (int)kColO + KW <= (int)kTmemCols, "TMEM budget");
-  static_assert(!PSEP || (!TWO && !LOSS) || LOSS, "separate P buffers: one-output kernels");
   static_assert(!TWO || (!SPLIT && RP == 64 && TN == 128 && NS == 2), "two-output kernels: fast mode, R <= 64");
   static_assert(TN == 64 || TN == 128, "tile width");
   static_assert(RP == 64 || RP == 128, "padded rank");
@@ -157,9 +133,10 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
   const uint32_t sF = sbase + L::kF, sG = sbase + L::kG, sV = sbase + L::kV;
   const uint32_t bar0 = sbase + L::kBar;
   auto BAR = [&](int i) { return bar0 + 8u * i; };
+  // S/P stage ring: S full (S-MMA -> ratio warps), P full (ratio warps -> O-MMA), P empty (O-MMA -> S-MMA: stage free)
   constexpr int B_FFULL = 0, B_FEMPTY = NF, B_GFULL = 2 * NF, B_GEMPTY = B_GFULL + NG, B_VFULL = B_GEMPTY + NG,
-                B_VEMPTY = B_VFULL + NV, B_SFULL = B_VEMPTY + NV, B_SEMPTY = B_SFULL + NS, B_PFULL = B_SEMPTY + NS,
-                B_PEMPTY = B_PFULL + NPB, B_OFULL = B_PEMPTY + NPB, B_OEMPTY = B_OFULL + 1;
+                B_VEMPTY = B_VFULL + NV, B_SFULL = B_VEMPTY + NV, B_PFULL = B_SFULL + NS, B_PEMPTY = B_PFULL + NS,
+                B_OFULL = B_PEMPTY + NS, B_OEMPTY = B_OFULL + 1;
   volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem_al + L::kTmemPtr);
   double* loss_slots = reinterpret_cast<double*>(smem_al + L::kLossSlots);      // [8 ratio warps][2]
 
@@ -170,8 +147,9 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
     for (int i = 0; i < NF; ++i) { ptx::mbar_init(BAR(B_FFULL + i), 1); ptx::mbar_init(BAR(B_FEMPTY + i), 1); }
     for (int i = 0; i < NG; ++i) { ptx::mbar_init(BAR(B_GFULL + i), 1); ptx::mbar_init(BAR(B_GEMPTY + i), 1); }
     for (int i = 0; i < NV; ++i) { ptx::mbar_init(BAR(B_VFULL + i), 1); ptx::mbar_init(BAR(B_VEMPTY + i), 4 * NRW); }
-    for (int i = 0; i < NS; ++i) { ptx::mbar_init(BAR(B_SFULL + i), 1); ptx::mbar_init(BAR(B_SEMPTY + i), 4 * NRW); }
-    for (int i = 0; i < NPB; ++i) { ptx::mbar_init(BAR(B_PFULL + i), 4 * NRW); ptx::mbar_init(BAR(B_PEMPTY + i), 1); }
+    for (int i = 0; i < NS; ++i) {
+      ptx::mbar_init(BAR(B_SFULL + i), 1); ptx::mbar_init(BAR(B_PFULL + i), 4 * NRW); ptx::mbar_init(BAR(B_PEMPTY + i), 1);
+    }
     ptx::mbar_init(BAR(B_OFULL), 1);
     ptx::mbar_init(BAR(B_OEMPTY), 4);
     ptx::fence_barrier_init();
@@ -190,30 +168,7 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
 
   if (warp == kCtl0) {
     // =========================== TMA producer: V tiles (the HBM stream) =================================
-    // HBM latency under load (~3 us) times the per-SM share of the bandwidth is more than the shared-memory ring
-    // can hold in flight, so the stream is staged through L2: tile t + kPfDist is prefetched into L2 (no smem,
-    // no barrier) while tile t is copied L2 -> smem into the ring.
     if (lane == 0) {
-      const int kPfDist = p.pf_dist;
-      int pf_item = blockIdx.x, pf_j = 0, pf_te = 0, pf_rb = 0;
-      bool pf_live = pf_item < total_items;
-      auto pf_load_item = [&]() {
-        pf_rb = pf_item % p.row_blocks;
-        const int chunk = pf_item / p.row_blocks;
-        pf_j = chunk * p.tiles_per_chunk;
-        pf_te = min(p.tiles, pf_j + p.tiles_per_chunk);
-      };
-      auto pf_issue_and_advance = [&]() {
-        if (!pf_live) return;
-        for (int vb = 0; vb < TN / 64; ++vb) ptx::tma_prefetch_l2_2d(&tmV, pf_j * TN + vb * 64, pf_rb * kTileM);
-        if (++pf_j >= pf_te) {
-          pf_item += gridDim.x;
-          pf_live = pf_item < total_items;
-          if (pf_live) pf_load_item();
-        }
-      };
-      if (pf_live) pf_load_item();
-      for (int k = 0; k < kPfDist; ++k) pf_issue_and_advance();
       uint32_t t = 0;
       for (int item = blockIdx.x; item < total_items; item += gridDim.x) {
         const int rb = item % p.row_blocks, chunk = item / p.row_blocks;
@@ -221,10 +176,7 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
         const int te = min(p.tiles, tb + p.tiles_per_chunk);
         for (int j = tb; j < te; ++j, ++t) {
           const uint32_t s = t % NV, ph = (t / NV) & 1;
-          if (kPfDist > 0) pf_issue_and_advance();
           ptx::mbar_wait(BAR(B_VEMPTY + s), ph ^ 1);
-          TC_TRACE(t, 7);
-          if (TC_KNOCK(32) && t >= (uint32_t)NV) { ptx::mbar_arrive(BAR(B_VFULL + s)); continue; }
           ptx::mbar_expect_tx(BAR(B_VFULL + s), L::kVBytes);
           for (int vb = 0; vb < TN / 64; ++vb)
             ptx::tma_load_2d(&tmV, BAR(B_VFULL + s), sV + s * L::kVBytes + vb * (kTileM * 128), j * TN + vb * 64,
@@ -248,7 +200,6 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
         for (int j = tb; j < te; ++j, ++t) {
           const uint32_t s = t % NG, ph = (t / NG) & 1;
           ptx::mbar_wait(BAR(B_GEMPTY + s), ph ^ 1);
-          TC_TRACE(t, 8);
           ptx::mbar_expect_tx(BAR(B_GFULL + s), L::kGBytes);
           for (int kb = 0; kb < KW / 64; ++kb)
             ptx::tma_load_2d(&tmG, BAR(B_GFULL + s), sG + s * L::kGBytes + kb * (TN * 128), kb * 64, j * TN);
@@ -261,7 +212,7 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
     // polls, descriptor arithmetic in uniform registers, tcgen05.mma issue: measured ~780 cycles per S or O step), so
     // one warp issuing both S and O produced one tile per ~1570 cycles and left the ratio warpgroups waiting for S.
     // This warp runs ahead with the S-MMAs, across work-item boundaries, bounded by the G ring and by the NS
-    // accumulator stages (p_empty: the O-MMA of the tile NS earlier has consumed the stage); warp 3 issues the O-MMAs as
+    // accumulator stages (P empty: the O-MMA of the tile NS earlier has consumed the stage); warp 3 issues the O-MMAs as
     // ratio tiles complete.  Each loop is warp-uniform; one elected lane issues tcgen05.mma / commit.
     {
       constexpr uint32_t idescS = ptx::idesc_f16(kTileM, TN, 0, 0);
@@ -270,8 +221,7 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
       constexpr int kTerms = SPLIT ? 3 : 1;
       constexpr int termF[3] = {0, 1, 0}, termG[3] = {0, 0, 1};
       uint32_t sg = 0, sg_ph = 0;                 // G stage / phase
-      uint32_t ss = 0, ss_ph = 0;                 // S stage / phase of its p_empty barrier
-      uint32_t ts = 0;                            // tile counter (trace only)
+      uint32_t ss = 0, ss_ph = 0;                 // S stage / phase of its P-empty barrier
       uint32_t it = 0;
       for (int item = blockIdx.x; item < total_items; item += gridDim.x, ++it) {
         const int tb = (item / p.row_blocks) * p.tiles_per_chunk;
@@ -282,13 +232,8 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
         const uint32_t fbase = sF + f_s * L::kFBytes;
         for (int j = 0; j < n; ++j) {
           if (lane == 0) {
-            TC_TRACE(ts, 0);
             ptx::mbar_wait(BAR(B_GFULL + sg), sg_ph);              // G tile landed
-            TC_TRACE(ts, 12);
-            // the stage is free: the O-MMA of the tile NS earlier consumed its P (alias layout) / the ratio warps have
-            // read the S of the tile NS earlier (P buffers of their own)
-            ptx::mbar_wait(BAR((PSEP && !LOSS ? B_SEMPTY : B_PEMPTY) + ss), ss_ph ^ 1);
-            TC_TRACE(ts, 1);
+            ptx::mbar_wait(BAR(B_PEMPTY + ss), ss_ph ^ 1);         // the O-MMA of the tile NS earlier consumed its P
           }
           __syncwarp();
           ptx::tc_fence_after();
@@ -297,7 +242,6 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
           if (ptx::elect_one()) {
 #pragma unroll
             for (int term = 0; term < kTerms; ++term) {
-              if (TC_KNOCK(16)) break;
               // operand halves (hi / lo) are RP/64 sub-blocks of 64 columns each; a k-step is 32 B inside a sub-block
 #pragma unroll
               for (int ks = 0; ks < RP / 16; ++ks) {
@@ -309,12 +253,10 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
             }
             ptx::mma_commit(BAR(B_SFULL + ss));
             if (j == n - 1) ptx::mma_commit(BAR(B_FEMPTY + f_s));  // last S of the item: its F block is free
-            TC_TRACE(ts, 13);
           }
           __syncwarp();
           if (++sg == NG) { sg = 0; sg_ph ^= 1; }
           if (++ss == NS) { ss = 0; ss_ph ^= 1; }
-          ++ts;
         }
       }
     }
@@ -323,9 +265,7 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
     {
       constexpr uint32_t idescO = ptx::idesc_f16(kTileM, KW, 0, 1);
       constexpr uint32_t descHi = ptx::smem_desc_hi_sw128(1024);
-      constexpr int NO = (PSEP && !LOSS) ? NP : NS;   // ring the O-MMAs walk: P buffers of their own, or the S/P stages
-      uint32_t og = 0, os = 0, os_ph = 0;         // G stage, P stage + p_full phase
-      uint32_t to = 0;                            // tile counter (trace only)
+      uint32_t og = 0, os = 0, os_ph = 0;         // G stage, S/P stage + phase of its P-full barrier
       uint32_t it = 0;
       for (int item = blockIdx.x; item < total_items; item += gridDim.x, ++it) {
         const int tb = (item / p.row_blocks) * p.tiles_per_chunk;
@@ -333,10 +273,8 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
         for (int j = 0; j < n; ++j) {
           const bool first = j == 0, last = j == n - 1;
           if (lane == 0) {
-            TC_TRACE(to, 5);
             ptx::mbar_wait(BAR(B_PFULL + os), os_ph);                              // ratio tile written
             if (first && !LOSS) ptx::mbar_wait(BAR(B_OEMPTY), (it & 1) ^ 1);       // epilogue drained O (none in LOSS mode)
-            TC_TRACE(to, 6);
           }
           __syncwarp();
           ptx::tc_fence_after();
@@ -349,31 +287,26 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
             // B = G tile as [K = 16 c-rows][N = KW] MN-major: 8-row groups 1024 B apart, 64-wide column blocks
             // (hi | lo, RP/64 blocks each) one sub-block (TN x 128 B) apart
             const uint32_t blo = ptx::smem_desc_lo(sG + og * L::kGBytes, TN * 128);
-            const uint32_t aP = PSEP ? tmem + kColP + os * (TN / 2) : tmem + kColS + os * TN;
+            const uint32_t aP = tmem + kColS + os * TN;
             if (ptx::elect_one()) {
 #pragma unroll
               for (int ks = 0; ks < TN / 16; ++ks) {
-                if (TC_KNOCK(8)) break;
-                // P k-step ks was written by ratio warpgroup ks / kKsPerWg: at the start of that warpgroup's S columns
-                // (alias layout) or packed in k order into the P buffer
+                // P k-step ks was written by ratio warpgroup ks / kKsPerWg, at the start of that warpgroup's S columns
                 constexpr int kKsPerWg = TN / 16 / NRW;
-                ptx::mma_ts(tmem + kColO, aP + (PSEP ? ks * 8 : (ks / kKsPerWg) * (TN / NRW) + (ks % kKsPerWg) * 8),
+                ptx::mma_ts(tmem + kColO, aP + (ks / kKsPerWg) * (TN / NRW) + (ks % kKsPerWg) * 8,
                             ptx::make_desc(blo + ks * 128, descHi), idescO, (first && ks == 0) ? 0u : 1u);
                 if (TWO)
                   ptx::mma_ts(tmem + kColO2, tmem + kColPp + os * 64 + ks * 8, ptx::make_desc(blo + ks * 128, descHi),
                               idescO, (first && ks == 0) ? 0u : 1u);
-                if (ks == 0) TC_TRACE(to, 15);
               }
               ptx::mma_commit(BAR(B_GEMPTY + og));     // G tile free (its S-MMA finished before the ratio tile existed)
               ptx::mma_commit(BAR(B_PEMPTY + os));     // S/P stage free
               if (last) ptx::mma_commit(BAR(B_OFULL));
-              TC_TRACE(to, 14);
             }
           }
           __syncwarp();
           if (++og == NG) og = 0;
-          if (++os == NO) { os = 0; os_ph ^= 1; }
-          ++to;
+          if (++os == NS) { os = 0; os_ph ^= 1; }
         }
       }
     }
@@ -451,7 +384,6 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
         ptx::tmem_ld16(tS + c * CW, sr);
 #pragma unroll
         for (int k = 0; k < NV4; ++k) {
-          if (TC_KNOCK(2)) { vv[k] = make_uint4(0x3c003c00u, 0x3c003c00u, 0x3c003c00u, 0x3c003c00u); continue; }
           const int col16 = c * NV4 + k;                                           // 16-byte column group of the tile (8 fp16)
           const uint32_t kx = (uint32_t)(col16 & 7) << 4;                          // compile-time per unrolled load
           asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];"
@@ -459,7 +391,7 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
                        : "r"((vT ^ kx) + (uint32_t)((col16 >> 3) * (kTileM * 128))));
         }
       };
-      auto compute_chunk = [&](uint32_t tS, uint32_t tP, int c, const uint32_t (&sr)[CW], const uint4 (&vv)[NV4]) {
+      auto compute_chunk = [&](uint32_t tS, int c, const uint32_t (&sr)[CW], const uint4 (&vv)[NV4]) {
         const uint32_t* vw = reinterpret_cast<const uint32_t*>(vv);
         uint32_t preg[CW / 2];
 #pragma unroll
@@ -491,15 +423,15 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
               // batched: 1 / x0 = x2 r0, 1 / x1 = x3 r1, 1 / x2 = x0 r0, 1 / x3 = x1 r1 with r = rcp(x_a x_b)
               float m0, m1;
               ptx::upk2(ptx::fma2(Xa, Xb, Z2), m0, m1);
-              const uint64_t Rr = ptx::pk2(TC_KNOCK(1) ? m0 : ptx::rcp_approx(m0), TC_KNOCK(1) ? m1 : ptx::rcp_approx(m1));
+              const uint64_t Rr = ptx::pk2(ptx::rcp_approx(m0), ptx::rcp_approx(m1));
               Ra = ptx::fma2(Rr, Xb, Z2);
               Rb = ptx::fma2(Rr, Xa, Z2);
             } else {
               float x0, x1, x2, x3;
               ptx::upk2(Xa, x0, x1);
               ptx::upk2(Xb, x2, x3);
-              Ra = ptx::pk2(TC_KNOCK(1) ? x0 : ptx::rcp_approx(x0), TC_KNOCK(1) ? x1 : ptx::rcp_approx(x1));
-              Rb = ptx::pk2(TC_KNOCK(1) ? x2 : ptx::rcp_approx(x2), TC_KNOCK(1) ? x3 : ptx::rcp_approx(x3));
+              Ra = ptx::pk2(ptx::rcp_approx(x0), ptx::rcp_approx(x1));
+              Rb = ptx::pk2(ptx::rcp_approx(x2), ptx::rcp_approx(x3));
             }
             Pa = ptx::fma2(Va, Ra, NEGPC);                                           // nmf.py:65, centred
             Pb = ptx::fma2(Vb, Rb, NEGPC);
@@ -510,20 +442,14 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
           preg[2 * qd] = ptx::pack_f16x2_sat(a0, a1);
           preg[2 * qd + 1] = ptx::pack_f16x2_sat(b0, b1);
         }
-        // P of warpgroup g goes over the S columns that warpgroup owns (and has already read): [g TN / NRW, ...), or into
-        // its k-ordered slice of the tile's own P buffer
-        const uint32_t dst = PSEP ? tP + c * (CW / 2) : tS + g * (TN / NRW) + (c - c_lo) * (CW / 2);
-        ptx::tmem_st8(dst, preg);
+        // P of warpgroup g goes over the S columns that warpgroup owns (and has already read): [g TN / NRW, ...)
+        ptx::tmem_st8(tS + g * (TN / NRW) + (c - c_lo) * (CW / 2), preg);
       };
       uint32_t st = 0, sv = 0, phS = 0, phV = 0;        // S stage and V slot of the tile being computed, phases of their full barriers
-      uint32_t pb = 0, phP = 0;                         // PSEP: P buffer of the tile being computed, phase of its empty barrier
       uint32_t tS = tS0, vT = sV + vrow;
-      const uint32_t tP0 = tmem + lane_addr + kColP;
       if (my_tiles > 0) {
-        if (q == 0 && lane == 0) TC_TRACE(0, 2);
         ptx::mbar_wait(BAR(B_VFULL), 0);                            // V tile landed (TMA -> this thread)
         ptx::mbar_wait(BAR(B_SFULL), 0);                            // S tile complete
-        if (q == 0 && lane == 0) TC_TRACE(0, 4);
         ptx::tc_fence_after();
         load_chunk(tS, vT, c_lo, sA, vA);
       }
@@ -534,8 +460,6 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
         if (st1 == NS) { st1 = 0; phS1 ^= 1; }
         if (sv1 == NV) { sv1 = 0; phV1 ^= 1; }
         const uint32_t tS1 = tS0 + st1 * TN, vT1 = sV + sv1 * L::kVBytes + vrow;
-        const uint32_t tP = tP0 + pb * (TN / 2);
-        if (PSEP) ptx::mbar_wait(BAR(B_PEMPTY + pb), phP ^ 1);      // the O-MMA of the tile NP earlier has consumed this buffer
 #pragma unroll
         for (int cc = 0; cc < kCpw; cc += 2) {
           const int c = c_lo + cc;
@@ -550,44 +474,27 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
           }
           ptx::tc_wait_ld();
           load_chunk(tS, vT, c + 1, sB, vB);
-          compute_chunk(tS, tP, c, sA, vA);
+          compute_chunk(tS, c, sA, vA);
           ptx::tc_wait_ld();
           if (!lastpair) {
             load_chunk(tS, vT, c + 2, sA, vA);
-          } else {
-            if (PSEP) {
-              // every S column of this tile is in registers (tcgen05.wait::ld above): hand the S stage back now, a chunk
-              // before the P tile is complete.  (Not the V slot: an ld.shared is only known to have landed once its
-              // result has been consumed.)
-              ptx::tc_fence_before();
-              __syncwarp();
-              if (lane == 0) ptx::mbar_arrive(BAR(B_SEMPTY + st));
-            }
-            if (more) {
-              if (g == 0 && q == 0 && lane == 0) TC_TRACE(tt + 1, 2);
-              if (!okV) ptx::mbar_wait(BAR(B_VFULL + sv1), phV1);
-              if (g == 0 && q == 0 && lane == 0) TC_TRACE(tt + 1, 3);
-              if (!okS) ptx::mbar_wait(BAR(B_SFULL + st1), phS1);
-              if (g == 0 && q == 0 && lane == 0) TC_TRACE(tt + 1, 4);
-              ptx::tc_fence_after();
-              load_chunk(tS1, vT1, c_lo, sA, vA);
-            }
+          } else if (more) {
+            if (!okV) ptx::mbar_wait(BAR(B_VFULL + sv1), phV1);
+            if (!okS) ptx::mbar_wait(BAR(B_SFULL + st1), phS1);
+            ptx::tc_fence_after();
+            load_chunk(tS1, vT1, c_lo, sA, vA);
           }
-          compute_chunk(tS, tP, c + 1, sB, vB);
+          compute_chunk(tS, c + 1, sB, vB);
         }
-        // hand the tile on: P complete (alias layout: this also frees the S stage once the O-MMA has run) + the V slot
-        if (lane == 0 && g == 0 && q == 0) TC_TRACE(tt, 10);
+        // hand the tile on: P complete (this also frees the S stage once the O-MMA has run) + the V slot
         ptx::tc_wait_st();
         ptx::tc_fence_before();
         __syncwarp();                  // every lane's P stores are complete and fenced, its V reads have returned
         if (lane == 0) {               // ONE arrival per warp (barrier counts = warps): 32x fewer mbarrier operations
-          ptx::mbar_arrive(BAR(B_PFULL + (PSEP ? pb : st)));
+          ptx::mbar_arrive(BAR(B_PFULL + st));
           ptx::mbar_arrive(BAR(B_VEMPTY + sv));
         }
-        if (lane == 0 && g == 0 && q == 0) TC_TRACE(tt, 9);
-        if (lane == 0 && g == NRW - 1 && q == 3) TC_TRACE(tt, 11);
         st = st1; phS = phS1; sv = sv1; phV = phV1; tS = tS1; vT = vT1;
-        if (PSEP && ++pb == (uint32_t)NP) { pb = 0; phP ^= 1; }
         if constexpr (FOLD) {                    // per-tile fp32 sums (TN / NRW elements per thread) into the double totals
           float b0, b1;
           ptx::upk2(FOLD_B, b0, b1);
@@ -607,11 +514,8 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
       for (int j = 0; j < n; ++j) {
         const uint32_t tt = t + j;
         const uint32_t s = tt % NV, st = tt % NS;
-        if (q == 0 && lane == 0) TC_TRACE(tt, 2);
         ptx::mbar_wait(BAR(B_VFULL + s), (tt / NV) & 1);              // V tile landed (TMA -> this thread)
-        if (q == 0 && lane == 0) TC_TRACE(tt, 3);
         ptx::mbar_wait(BAR(B_SFULL + st), (tt / NS) & 1);       // S tile complete
-        if (q == 0 && lane == 0) TC_TRACE(tt, 4);
         ptx::tc_fence_after();
         const uint32_t vrow = sV + s * L::kVBytes + row * 128;
         {
@@ -624,7 +528,6 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
           const uint32_t vsub = vrow + (c4 >> 1) * (kTileM * 128);
 #pragma unroll
           for (int k = 0; k < 4; ++k) {
-            if (TC_KNOCK(2)) { vv[k] = make_uint4(0x3c003c00u, 0x3c003c00u, 0x3c003c00u, 0x3c003c00u); continue; }
             const uint32_t chunk16 = (uint32_t)((c4 & 1) * 4 + k) ^ (uint32_t)(row & 7);
             asm volatile("ld.shared.v4.u32 {%0, %1, %2, %3}, [%4];"
                          : "=r"(vv[k].x), "=r"(vv[k].y), "=r"(vv[k].z), "=r"(vv[k].w)
@@ -722,7 +625,6 @@ tc_contract_kernel(const __grid_constant__ CUtensorMap tmF, const __grid_constan
           ptx::mbar_arrive(BAR(B_PFULL + st));
           ptx::mbar_arrive(BAR(B_VEMPTY + s));
         }
-        if (q == 0 && lane == 0) TC_TRACE(tt, 9);
       }
       t += n;
     }
@@ -997,12 +899,7 @@ tc_apply_kernel(TcApplyArgs a) {
           num = fmaf(kap, klden, num);                          // the kernel accumulated sum (P - kappa) G
           pos = klden;                                          // nmf.py:368-369 / :381-382
         }
-        const float neg = fmaxf(num, 0.f) + kEps;              // nmf.py:78
-        if (a.l1 > 0.f) pos += a.l1;                            // nmf.py:85-86
-        if (a.l2 > 0.f) pos = fmaf(a.l2, v, pos);               // nmf.py:87-88
-        float mult = neg / pos;                                 // nmf.py:89
-        if (a.gamma != 1.0f) mult = powf(mult, a.gamma);        // nmf.py:90-91
-        v *= mult;                                              // nmf.py:92
+        v = mu_step(v, num, pos, a.l1, a.l2, a.gamma);
         a.param[idx] = v;
       }
       cs += v;
@@ -1012,72 +909,6 @@ tc_apply_kernel(TcApplyArgs a) {
   sh[rg][r] = cs;
   __syncthreads();
   if (threadIdx.x < 128) a.cs_part[(int64_t)blockIdx.x * 128 + r] = sh[0][r] + sh[1][r];
-  for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-  if ((threadIdx.x & 31) == 0 && mx > 0.f) atomicMax(a.absmax, __float_as_uint(mx));
-}
-
-// Vectorised variant for R % 4 == 0: one thread owns 4 consecutive rank lanes (float4) of a row; a 256-thread block
-// covers 256 / (R/4) rows per pass.  Same outputs as tc_apply_kernel.
-__global__ void __launch_bounds__(256)
-tc_apply_vec4_kernel(TcApplyArgs a) {
-  __shared__ float4 sh[256];
-  const int lanes = a.R >> 2;                    // threads per row
-  const int rows_per_pass = 256 / lanes;
-  const int rl = threadIdx.x / lanes, q = threadIdx.x - rl * lanes;      // row slot, rank quad
-  const int64_t row0 = (int64_t)blockIdx.x * a.rpb;
-  const int64_t row1 = min(a.rows, row0 + a.rpb);
-  float4 cs = make_float4(0.f, 0.f, 0.f, 0.f);
-  float mx = 0.f;
-  if (rl < rows_per_pass) {
-    float4 kd = make_float4(1.f, 1.f, 1.f, 1.f);
-    float kap = 0.f;
-    if (a.apply && !a.den) { kd = *reinterpret_cast<const float4*>(a.kl_den + 4 * q); kap = *a.kappa; }
-    for (int64_t row = row0 + rl; row < row1; row += rows_per_pass) {
-      float4* pp = reinterpret_cast<float4*>(a.param + row * a.R) + q;
-      float4 v = *pp;
-      if (a.apply) {
-        float4 num = make_float4(0.f, 0.f, 0.f, 0.f);
-        for (int ch = 0; ch < a.nchunks; ++ch) {
-          const float4 t = *(reinterpret_cast<const float4*>(a.num + ch * a.chunk_stride + row * a.Rp) + q);
-          num.x += t.x; num.y += t.y; num.z += t.z; num.w += t.w;
-        }
-        float4 dsum = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (a.den) {
-          for (int ch = 0; ch < a.nchunks; ++ch) {
-            const float4 t = *(reinterpret_cast<const float4*>(a.den + ch * a.chunk_stride + row * a.Rp) + q);
-            dsum.x += t.x; dsum.y += t.y; dsum.z += t.z; dsum.w += t.w;
-          }
-        }
-        float vv[4] = {v.x, v.y, v.z, v.w}, nn[4] = {num.x, num.y, num.z, num.w}, dd[4] = {kd.x, kd.y, kd.z, kd.w};
-        const float ds[4] = {dsum.x, dsum.y, dsum.z, dsum.w};
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          const float n = a.den ? nn[i] : fmaf(kap, dd[i], nn[i]);  // beta == 1: the kernel accumulated sum (P - kappa) G
-          const float neg = fmaxf(n, 0.f) + kEps;                   // nmf.py:78
-          float pos = a.den ? fmaxf(ds[i], 0.f) + kEps : dd[i];     // nmf.py:83 | nmf.py:368-369 / :381-382
-          if (a.l1 > 0.f) pos += a.l1;                              // nmf.py:85-86
-          if (a.l2 > 0.f) pos = fmaf(a.l2, vv[i], pos);             // nmf.py:87-88
-          float mult = neg / pos;                                   // nmf.py:89
-          if (a.gamma != 1.0f) mult = powf(mult, a.gamma);          // nmf.py:90-91
-          vv[i] *= mult;                                            // nmf.py:92
-        }
-        v = make_float4(vv[0], vv[1], vv[2], vv[3]);
-        *pp = v;
-      }
-      cs.x += v.x; cs.y += v.y; cs.z += v.z; cs.w += v.w;
-      mx = fmaxf(fmaxf(mx, fmaxf(v.x, v.y)), fmaxf(v.z, v.w));
-    }
-  }
-  sh[threadIdx.x] = cs;
-  __syncthreads();
-  if (threadIdx.x < lanes) {
-    float4 t = make_float4(0.f, 0.f, 0.f, 0.f);
-    for (int k = 0; k < rows_per_pass; ++k) {
-      const float4 u = sh[k * lanes + threadIdx.x];
-      t.x += u.x; t.y += u.y; t.z += u.z; t.w += u.w;
-    }
-    *(reinterpret_cast<float4*>(a.cs_part + (int64_t)blockIdx.x * 128) + threadIdx.x) = t;
-  }
   for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
   if ((threadIdx.x & 31) == 0 && mx > 0.f) atomicMax(a.absmax, __float_as_uint(mx));
 }
@@ -1269,14 +1100,7 @@ tc_apply_eu_kernel(TcApplyArgs a, const float* __restrict__ gram) {
         if (r >= R) continue;
         const float den = acc[i][j];
         const float num = fmaf(kap, den, numv[i][j]);            // numerator = (V - kappa S) G + kappa S G
-        float v = fs[(ty * 4 + i) * FP + r];
-        const float neg = fmaxf(num, 0.f) + kEps;                // nmf.py:78
-        float pos = fmaxf(den, 0.f) + kEps;                      // nmf.py:83
-        if (a.l1 > 0.f) pos += a.l1;                              // nmf.py:85-86
-        if (a.l2 > 0.f) pos = fmaf(a.l2, v, pos);                 // nmf.py:87-88
-        float mult = neg / pos;                                   // nmf.py:89
-        if (a.gamma != 1.0f) mult = powf(mult, a.gamma);          // nmf.py:90-91 (gamma == 1 for beta 2)
-        v *= mult;                                                // nmf.py:92
+        const float v = mu_step(fs[(ty * 4 + i) * FP + r], num, fmaxf(den, 0.f) + kEps, a.l1, a.l2, a.gamma);   // nmf.py:83
         a.param[row * R + r] = v;
         cs[j] += v;
         mx = fmaxf(mx, v);
@@ -1392,7 +1216,8 @@ tc_finish_kernel(const float* __restrict__ x, int64_t rows, int R, __half* __res
 }
 
 // ---- ratio stage + operand refresh in ONE cooperative kernel (R % 4 == 0; beta != 2) ------------------------------------
-// Phase 1 = tc_apply_vec4_kernel (nmf.py:78-92 in place, per-block column sums, global max); grid barrier; phase 2 = the
+// Phase 1 = the ratio stage of tc_apply_kernel with one thread per four consecutive rank lanes (nmf.py:78-92 in place,
+// per-block column sums, global max); grid barrier; phase 2 = the
 // fp16 operand copy with the exponent from that max (rows re-read from L2), while block 0 folds the column sums in fixed
 // order and publishes colsum / kappa / exponents.  Replaces two launches, one pass over the factor and the ticket
 // protocol of tc_finish_kernel; the W side also gets 2 x #SM blocks instead of rows / 64.
@@ -1489,13 +1314,8 @@ tc_apply_finish_kernel(TcApplyArgs a, TcFinishArgs f) {
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
           const float n = a.den ? nn[i] : fmaf(kap, dd[i], nn[i]);  // beta == 1: the kernel accumulated sum (P - kappa) G
-          const float neg = fmaxf(n, 0.f) + kEps;                   // nmf.py:78
-          float pos = a.den ? fmaxf(ds[i], 0.f) + kEps : dd[i];     // nmf.py:83 | nmf.py:368-369 / :381-382
-          if (a.l1 > 0.f) pos += a.l1;                              // nmf.py:85-86
-          if (a.l2 > 0.f) pos = fmaf(a.l2, vv[i], pos);             // nmf.py:87-88
-          float mult = neg / pos;                                   // nmf.py:89
-          if (a.gamma != 1.0f) mult = powf(mult, a.gamma);          // nmf.py:90-91
-          vv[i] *= mult;                                            // nmf.py:92
+          const float pos = a.den ? fmaxf(ds[i], 0.f) + kEps : dd[i];   // nmf.py:83 | nmf.py:368-369 / :381-382
+          vv[i] = mu_step(vv[i], n, pos, a.l1, a.l2, a.gamma);
         }
         v = make_float4(vv[0], vv[1], vv[2], vv[3]);
         *pp = v;
@@ -1807,41 +1627,19 @@ struct TcState {
   CUtensorMap tmWg, tmHg;           // factors as the column factor G: box 64 x TN
   Plan plan_w, plan_h;
   uint32_t upd[2] = {0, 0};         // per-factor update counter (selects the absmax slot)
-  // one MU iteration (W update + H update) captured as a CUDA graph, per absmax-slot parity pair
-  cudaGraphExec_t gexec[4] = {nullptr, nullptr, nullptr, nullptr};
-  int gkernels = 0;                 // kernels per captured iteration (for the launch counter)
-  const float* gW = nullptr; const float* gH = nullptr;
-  double gargs[4] = {0, 0, 0, 0};   // beta, gamma, l1, l2 the graphs were captured with
-  bool gwarm = false;               // one eager iteration has run with these arguments
-  cudaStream_t gstream = nullptr;   // capture / replay stream (the caller's may be the legacy default stream, which cannot capture)
-  cudaEvent_t gev_in = nullptr, gev_out = nullptr;
   bool dirty_w = true, dirty_h = true, has_target = false;
-  // Environment knobs, read once in tc_create.  Product build: NMFB200_CENTER=0 (diagnostic: kappa centring off, see
-  // tools/bias_probe.py), NMFB200_GRAPH=1 (CUDA-graph replay of tc_iterate), NMFB200_TC_CHECK=1 (watchdog check after
-  // every tc_contract_only).  Tuning build (-DNMFB200_TRACE) only: NMFB200_TC_VARIANT, NMFB200_TC_PF, NMFB200_TC_KNOCK,
-  // NMFB200_TC_PARK, NMFB200_TC_TRACE=<file>.
+  // Environment knobs, read once in tc_create: NMFB200_CENTER=0 (diagnostic: kappa centring off, see
+  // tools/bias_probe.py), NMFB200_TC_CHECK=1 (watchdog check after every tc_contract_only).
   int center = 1;
-  bool use_graph = false, check_each = false;
-  int pf_dist = 0;                  // L2 prefetch distance of the V stream in tiles (measured: no gain; 0 = off)
-  int variant = 0;                  // pipeline configuration variant
-  int knock = 0;                    // knock-out mask (tools/tc_knock.py)
-  long long* trace = nullptr;       // event timestamps of CTA 0 (tools/tc_trace.py)
-  std::string trace_path;
+  bool check_each = false;
   float* kappa = nullptr;           // device scalar
   float* zero = nullptr;            // device scalar 0 (kappa of an already complete numerator)
   int coop_blocks = 0;              // co-resident blocks of the fused tail kernel (cooperative launch), 0 = unavailable
-  bool psep = false;                // R <= 64 f16 kernel: P buffers of their own (NMFB200_TC_PSEP=1; staged, see DESIGN.md)
-  bool fused_tail = false;          // ratio stage + operand refresh in one cooperative kernel (NMFB200_FUSED_TAIL=0: two kernels)
 };
 
 bool tc_shape_supported(int64_t N, int64_t C, int64_t R) {
   // the conversion kernel walks 64-row slabs on gridDim.y (<= 65535): taller targets take the fp32 kernels
   return R >= 1 && R <= 128 && N >= 1 && C >= 1 && N <= 65535ll * 64 && C < (1ll << 31);
-}
-
-static void drop_graphs(TcState* s) {
-  for (auto& g : s->gexec) { if (g) cudaGraphExecDestroy(g); g = nullptr; }
-  s->gwarm = false;
 }
 
 void tc_peer_release(TcState* s) {
@@ -1857,13 +1655,9 @@ void tc_peer_release(TcState* s) {
 void tc_destroy(TcState* s) {
   if (!s) return;      // the caller (capi.cu: free_ctx) has selected s->device
   tc_peer_release(s);
-  drop_graphs(s);
-  if (s->gstream) cudaStreamDestroy(s->gstream);
-  if (s->gev_in) cudaEventDestroy(s->gev_in);
-  if (s->gev_out) cudaEventDestroy(s->gev_out);
   cudaFree(s->V16); cudaFree(s->Vt16); cudaFree(s->W16); cudaFree(s->H16); cudaFree(s->part); cudaFree(s->part2); cudaFree(s->gram); cudaFree(s->gram_part);
   cudaFree(s->colsum); cudaFree(s->cs_part); cudaFree(s->cs_super); cudaFree(s->ticket); cudaFree(s->absmax); cudaFree(s->exps);
-  cudaFree(s->vpart); cudaFree(s->vconst); cudaFree(s->vlossy); cudaFree(s->loss_part); cudaFree(s->vbeta); cudaFree(s->vbeta_part); cudaFree(s->kappa); cudaFree(s->zero); cudaFree(s->trace);
+  cudaFree(s->vpart); cudaFree(s->vconst); cudaFree(s->vlossy); cudaFree(s->loss_part); cudaFree(s->vbeta); cudaFree(s->vbeta_part); cudaFree(s->kappa); cudaFree(s->zero);
   delete s;
 }
 
@@ -1875,29 +1669,13 @@ int tc_create(TcState** out, int device, int64_t N, int64_t C, int64_t R, bool s
   s->KW = split ? 2 * s->Rp : s->Rp;
   s->TN = (split && s->Rp == 128) ? 64 : 128;   // 64-column tiles only where 128 do not fit (measured slower: MMA issue rate)
   if (const char* e = getenv("NMFB200_CENTER")) s->center = atoi(e);
-  s->use_graph = getenv("NMFB200_GRAPH") != nullptr;
   s->check_each = getenv("NMFB200_TC_CHECK") != nullptr;
-  if (const char* e = getenv("NMFB200_TC_PSEP")) s->psep = atoi(e) != 0;
-#ifdef NMFB200_TRACE
-  if (const char* e = getenv("NMFB200_TC_VARIANT")) s->variant = atoi(e);
-  if (const char* e = getenv("NMFB200_TC_PF")) s->pf_dist = atoi(e);
-  if (const char* e = getenv("NMFB200_TC_KNOCK")) s->knock = atoi(e);
-  {
-    const unsigned int park = getenv("NMFB200_TC_PARK") ? (unsigned)atoi(getenv("NMFB200_TC_PARK")) : 0u;   // default: parked polls; 2 = plain poll loop; > 2 = nanosleep(n) back-off
-    cudaMemcpyToSymbol(ptx::g_tune_park, &park, sizeof(park));
-  }
-  if (const char* e = getenv("NMFB200_TC_TRACE")) {
-    s->trace_path = e;
-    if (cudaMalloc(&s->trace, 256 * 16 * sizeof(long long)) != cudaSuccess) s->trace = nullptr;
-  }
-#endif
   s->ldc = round_up(C, 8);
   s->ldn = round_up(N, 8);
   cudaDeviceProp prop;
   NMF_CUDA_CHECK(cudaGetDeviceProperties(&prop, device));
   s->num_sms = prop.multiProcessorCount;
   if (prop.major != 10) { delete s; set_error("the tensor-core path needs an sm_100 device"); return 1; }
-  if (s->variant == 1 && split && s->Rp == 64) s->TN = 64;
   {
     int coop = 0, per_sm = 0;
     cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, device);
@@ -1907,8 +1685,6 @@ int tc_create(TcState** out, int device, int64_t N, int64_t C, int64_t R, bool s
       s->coop_blocks = per_sm * s->num_sms;
       if (s->coop_blocks > 1024) s->coop_blocks = 1024;      // cs_part capacity
     }
-    const char* e = getenv("NMFB200_FUSED_TAIL");
-    s->fused_tail = s->coop_blocks > 0 && !(e && atoi(e) == 0);
   }
   s->plan_w = make_plan(C, N, s->num_sms, s->TN);
   s->plan_h = make_plan(N, C, s->num_sms, s->TN);
@@ -1983,7 +1759,6 @@ int tc_set_target(TcState* s, const float* V, int64_t ldv, const float* minmax_d
   NMF_LAUNCH_CHECK();
   s->has_target = true;
   s->Vsrc = V; s->ldv = ldv; s->vbeta_for = 1.0;
-  drop_graphs(s);
   s->dirty_w = s->dirty_h = true;      // exps[3] depends on sum(V)
   return 0;
 }
@@ -2034,7 +1809,7 @@ int apply_and_finish(TcState* s, int which, float* param, bool apply, const Plan
   a.gamma = (float)gamma; a.l1 = (float)l1; a.l2 = (float)l2;
   a.cs_part = s->cs_part; a.absmax = slot; a.apply = apply ? 1 : 0; a.kappa = reduced ? s->zero : s->kappa;
   if (peer) {
-    if (!((s->R & 3) == 0 && s->fused_tail)) { set_error("internal: peer W update needs the fused ratio-stage kernel"); return 1; }
+    if (!((s->R & 3) == 0 && s->coop_blocks > 0)) { set_error("internal: peer W update needs the fused ratio-stage kernel"); return 1; }
     // the ranks' slots of THIS rank's block for this iteration's parity (every rank pushed its packed partial into them)
     for (int p = 0; p < s->peer_world; ++p)
       a.peers[p] = reinterpret_cast<const float*>(s->peer_block) + 64 +
@@ -2042,7 +1817,7 @@ int apply_and_finish(TcState* s, int which, float* param, bool apply, const Plan
     a.npeers = s->peer_world; a.flags = reinterpret_cast<const unsigned int*>(s->peer_block);
     a.flag_target = s->peer_iter; a.peer_err = s->peer_err;
   }
-  if ((s->R & 3) == 0 && !(apply && beta == 2.0 && !reduced) && s->fused_tail) {
+  if ((s->R & 3) == 0 && !(apply && beta == 2.0 && !reduced) && s->coop_blocks > 0) {
     // one cooperative launch: ratio stage, grid barrier, operand copy + scalars
     const int lanes = (int)s->R >> 2, rows_per_pass = 256 / lanes;
     int64_t g = ceil_div(rows, rows_per_pass);
@@ -2089,8 +1864,6 @@ int apply_and_finish(TcState* s, int which, float* param, bool apply, const Plan
       }
       tc_apply_eu_kernel<8><<<blocks, 256, eu_smem, st>>>(a, s->gram);
     }
-  } else if ((s->R & 3) == 0) {
-    tc_apply_vec4_kernel<<<blocks, 256, 0, st>>>(a);
   } else {
     tc_apply_kernel<<<blocks, 256, 0, st>>>(a);
   }
@@ -2128,7 +1901,7 @@ int ensure_synced(TcState* s, const float* W, const float* H, double beta, cudaS
 
 template <class C, int BM, bool LOSS, bool FOLD = false>
 int launch_contract_t(TcState* s, int which, double beta, cudaStream_t st) {
-  using L = SmemLayout<C::KW, C::TN, C::NF, C::NG, C::NV, C::NS, C::NP>;
+  using L = SmemLayout<C::KW, C::TN, C::NF, C::NG, C::NV, C::NS>;
   static_assert(L::kTotal + 1024 <= 232448, "shared memory budget (227 KB)");
   auto kern = tc_contract_kernel<C, BM, LOSS, FOLD>;
   if (!LOSS) s->w_pending = false;       // every update contraction overwrites the partial numerators
@@ -2151,10 +1924,6 @@ int launch_contract_t(TcState* s, int which, double beta, cudaStream_t st) {
   p.eg = which == 0 ? 2 : 1;
   p.loss_part = s->loss_part;
   p.kappa = s->kappa;
-  p.trace = s->trace;
-  p.knock = s->knock;
-  p.pf_dist = s->pf_dist;
-  if (s->trace) cudaMemsetAsync(s->trace, 0, 256 * 16 * sizeof(long long), st);
   const int items = pl.row_blocks * pl.nchunks;
   const int grid = items < s->num_sms ? items : s->num_sms;
   if (which == 0)
@@ -2168,34 +1937,18 @@ int launch_contract_t(TcState* s, int which, double beta, cudaStream_t st) {
 // Kernel configurations <RP, SPLIT, TN, NF, NG, NV, NS> (224 KB of shared memory each).  Tuning notes in
 // profiles/README.md and DESIGN.md 4.1: the V ring must keep >= 3 tiles (>= 64 KB) in flight to cover HBM latency, the G
 // ring needs >= 4 stages (a G tile stays resident from its S-MMA to its O-MMA); deeper G rings (5, 6) changed nothing.
-using CfgFast64 = Cfg<64, false, 128, 2, 4, 4, 2, 2, 3>;   // F 2x16 | G 4x16 | V 4x32 KB ; TMEM S 2x128 + P 3x64 + O 64
-using CfgFast64A = Cfg<64, false, 128, 2, 4, 4, 3, 2>;     // round-1 layout (P over S, 3 stages): NMFB200_TC_PSEP=0, A/B only
+using CfgFast64 = Cfg<64, false, 128, 2, 4, 4, 3>;       // F 2x16 | G 4x16 | V 4x32 KB     ; TMEM 3x128 + 64
 using CfgSplit64 = Cfg<64, true, 128, 1, 3, 3, 3>;       // F 32 | G 3x32 | V 3x32 KB     ; TMEM 3x128 + 128
-using CfgSplit64N = Cfg<64, true, 64, 1, 6, 6, 4>;       // (variant 1) 64-column tiles, deeper rings: slower
 using CfgFast128 = Cfg<128, false, 128, 1, 3, 3, 3>;     // F 32 | G 3x32 | V 3x32 KB     ; TMEM 3x128 + 128
 using CfgSplit128 = Cfg<128, true, 64, 1, 3, 4, 4>;      // F 64 | G 3x32 | V 4x16 KB     ; TMEM 4x64 + 256
-
-#ifdef NMFB200_TRACE    // tuning build: ring-depth experiments (NMFB200_TC_VARIANT = 4, 5, 6)
-using CfgFast64V4 = Cfg<64, false, 128, 1, 5, 4, 3>;
-using CfgFast64V5 = Cfg<64, false, 128, 1, 6, 3, 3>;
-using CfgFast64V6 = Cfg<64, false, 128, 1, 3, 5, 3>;
-#endif
+using CfgLoss64 = Cfg<64, false, 128, 2, 4, 4, 2>;       // loss sums, R <= 64 fast: F 2x16 | G 4x16 | V 4x32 KB ; TMEM 2x128
 using CfgTwo64 = Cfg<64, false, 128, 2, 3, 4, 2>;        // beta != 1: F 2x16 | G 3x16 | V 4x32 KB ; TMEM 2x128 + 128 + 2x64
 
 // one-output kernels (beta 1: BM = kBmKL, beta 2: BM = kBmEU) over the configuration of this context
 template <int BM>
 int launch_contract_one(TcState* s, int which, double beta, cudaStream_t st) {
-#ifdef NMFB200_TRACE
-  if (s->Rp == 64 && BM == kBmKL && !s->split) {
-    if (s->variant == 4) return launch_contract_t<CfgFast64V4, BM, false>(s, which, beta, st);
-    if (s->variant == 5) return launch_contract_t<CfgFast64V5, BM, false>(s, which, beta, st);
-    if (s->variant == 6) return launch_contract_t<CfgFast64V6, BM, false>(s, which, beta, st);
-  }
-#endif
   if (s->Rp == 64) {
-    if (!s->split && !s->psep) return launch_contract_t<CfgFast64A, BM, false>(s, which, beta, st);
     if (!s->split) return launch_contract_t<CfgFast64, BM, false>(s, which, beta, st);
-    if (s->TN == 64) return launch_contract_t<CfgSplit64N, BM, false>(s, which, beta, st);
     return launch_contract_t<CfgSplit64, BM, false>(s, which, beta, st);
   }
   if (!s->split) return launch_contract_t<CfgFast128, BM, false>(s, which, beta, st);
@@ -2204,18 +1957,14 @@ int launch_contract_one(TcState* s, int which, double beta, cudaStream_t st) {
 
 // beta 1, W orientation, loss sums folded in (fast, non-split configurations)
 int launch_contract_w_fold(TcState* s, cudaStream_t st) {
-  if (s->Rp == 64) {
-    if (!s->psep) return launch_contract_t<CfgFast64A, kBmKL, false, true>(s, 0, 1.0, st);
-    return launch_contract_t<CfgFast64, kBmKL, false, true>(s, 0, 1.0, st);
-  }
+  if (s->Rp == 64) return launch_contract_t<CfgFast64, kBmKL, false, true>(s, 0, 1.0, st);
   return launch_contract_t<CfgFast128, kBmKL, false, true>(s, 0, 1.0, st);
 }
 
 template <int BM>
 int launch_loss_bm(TcState* s, double beta, cudaStream_t st) {
   if (s->Rp == 64) {
-    if (!s->split) return launch_contract_t<CfgFast64, BM, true>(s, 1, beta, st);
-    if (s->TN == 64) return launch_contract_t<CfgSplit64N, BM, true>(s, 1, beta, st);
+    if (!s->split) return launch_contract_t<CfgLoss64, BM, true>(s, 1, beta, st);
     return launch_contract_t<CfgSplit64, BM, true>(s, 1, beta, st);
   }
   if (!s->split) return launch_contract_t<CfgFast128, BM, true>(s, 1, beta, st);
@@ -2266,63 +2015,10 @@ int tc_update_h(TcState* s, const float* W, float* H, double beta, double gamma,
 
 int tc_iterate(TcState* s, float* W, float* H, double beta, double gamma, double l1, double l2, int n_iter,
                cudaStream_t st) {
-  if (n_iter <= 0) return 0;
-  if (s->gW != W || s->gH != H || s->gargs[0] != beta || s->gargs[1] != gamma || s->gargs[2] != l1 || s->gargs[3] != l2) {
-    drop_graphs(s);
-    s->gW = W; s->gH = H; s->gargs[0] = beta; s->gargs[1] = gamma; s->gargs[2] = l1; s->gargs[3] = l2;
-  }
-  // CUDA-graph replay of the iteration is opt-in (NMFB200_GRAPH=1): measured no gain at cfg2 -- the stream is never
-  // launch-bound (profiles/README.md) -- so the default keeps plain stream-ordered launches.
-  const bool use_graph = s->use_graph && s->trace == nullptr;
-  cudaStream_t user = st;
-  if (use_graph) {
-    // run on an engine-owned stream, fenced against the caller's stream with events
-    if (!s->gstream) {
-      NMF_CUDA_CHECK(cudaStreamCreateWithFlags(&s->gstream, cudaStreamNonBlocking));
-      NMF_CUDA_CHECK(cudaEventCreateWithFlags(&s->gev_in, cudaEventDisableTiming));
-      NMF_CUDA_CHECK(cudaEventCreateWithFlags(&s->gev_out, cudaEventDisableTiming));
-    }
-    NMF_CUDA_CHECK(cudaEventRecord(s->gev_in, user));
-    NMF_CUDA_CHECK(cudaStreamWaitEvent(s->gstream, s->gev_in, 0));
-    st = s->gstream;
-  }
-  int rc = ensure_synced(s, W, H, beta, st);        // graphs assume clean operand copies
-  if (rc) return rc;
-  if (beta != 1.0 && !s->part2) NMF_CUDA_CHECK(cudaMalloc(&s->part2, (size_t)s->part_floats * 4));
   for (int i = 0; i < n_iter; ++i) {
-    const int key = (int)((s->upd[0] & 1u) * 2u + (s->upd[1] & 1u));
-    if (use_graph && s->gwarm && s->gexec[key]) {
-      s->w_pending = false;                          // the replayed iteration runs its own W contraction
-      NMF_CUDA_CHECK(cudaGraphLaunch(s->gexec[key], st));
-      s->upd[0]++; s->upd[1]++;
-      count_launch(s->gkernels);
-      continue;
-    }
-    const bool capture = use_graph && s->gwarm;      // the first iteration runs eagerly (lazy module loads, attributes)
-    cudaGraph_t graph = nullptr;
-    const int64_t before = launch_counter();
-    if (capture) NMF_CUDA_CHECK(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-    rc = tc_update_w(s, W, H, beta, gamma, l1, l2, st);
+    int rc = tc_update_w(s, W, H, beta, gamma, l1, l2, st);
     if (rc == 0) rc = tc_update_h(s, W, H, beta, gamma, l1, l2, st);
-    if (capture) {
-      cudaError_t e = cudaStreamEndCapture(st, &graph);
-      if (rc == 0 && e != cudaSuccess) { set_error(std::string("cudaStreamEndCapture: ") + cudaGetErrorString(e)); rc = 2; }
-      if (rc == 0) {
-        e = cudaGraphInstantiate(&s->gexec[key], graph, 0);
-        if (e != cudaSuccess) { set_error(std::string("cudaGraphInstantiate: ") + cudaGetErrorString(e)); rc = 2; }
-      }
-      if (graph) cudaGraphDestroy(graph);
-      if (rc) { drop_graphs(s); return rc; }
-      s->gkernels = (int)(launch_counter() - before);
-      NMF_CUDA_CHECK(cudaGraphLaunch(s->gexec[key], st));      // capture records, it does not execute
-    } else {
-      if (rc) return rc;
-      s->gwarm = true;
-    }
-  }
-  if (use_graph) {
-    NMF_CUDA_CHECK(cudaEventRecord(s->gev_out, s->gstream));
-    NMF_CUDA_CHECK(cudaStreamWaitEvent(user, s->gev_out, 0));
+    if (rc) return rc;
   }
   return 0;
 }
@@ -2367,7 +2063,7 @@ int tc_w_apply(TcState* s, float* W, const float* reduced, double beta, double g
 // between; slots alternate by iteration parity (a rank can be at most one W update ahead of the slowest: its next push needs
 // every rank's counter of the update in between, which that rank publishes after it has read the previous slots).
 bool tc_peer_supported(const TcState* s, double beta) {
-  return (s->R & 3) == 0 && s->fused_tail && tc_supports_partial(s, beta);
+  return (s->R & 3) == 0 && s->coop_blocks > 0 && tc_supports_partial(s, beta);
 }
 
 int tc_peer_alloc(TcState* s, void* handle_out) {
@@ -2473,23 +2169,11 @@ int tc_contract_only(TcState* s, const float* W, const float* H, int which, doub
   if (rc == 0 && s->check_each) {
     if (tc_check_wait_abort(st) > 0) { set_error("mbarrier wait aborted (protocol bug)"); return 2; }
   }
-  if (rc == 0 && s->trace) {
-    std::vector<long long> h(256 * 16);
-    cudaMemcpyAsync(h.data(), s->trace, h.size() * sizeof(long long), cudaMemcpyDeviceToHost, st);
-    cudaStreamSynchronize(st);
-    if (FILE* f = fopen(s->trace_path.c_str(), "w")) {
-      for (int t = 0; t < 256; ++t) {
-        for (int k = 0; k < 16; ++k) fprintf(f, "%lld ", h[t * 16 + k]);
-        fprintf(f, "\n");
-      }
-      fclose(f);
-    }
-  }
   return rc;
 }
 
 bool tc_supports_loss_prefetch(const TcState* s, double beta) {
-  return beta == 1.0 && !s->split && s->trace == nullptr;
+  return beta == 1.0 && !s->split;
 }
 
 // The loss at the current factors from the W update's own contraction (beta 1): one pass over V yields both the loss sums and

@@ -20,7 +20,6 @@ apply_update_kernel(ApplyArgs a) {
     num *= sc;
     if (a.kappa) num = fmaf(*a.kappa, a.kappa_vec[r], num);
     const float p = a.param[idx];
-    float neg = fmaxf(num, 0.f) + kEps;                      // nmf.py:78
     float pos;
     if (a.den) {
       float den = 0.f;
@@ -30,11 +29,7 @@ apply_update_kernel(ApplyArgs a) {
     } else {
       pos = a.kl_den[r];                                     // nmf.py:368-369 / :381-382 (no relu, no eps)
     }
-    if (a.l1 > 0.f) pos += a.l1;                             // nmf.py:85-86
-    if (a.l2 > 0.f) pos = fmaf(a.l2, p, pos);                // nmf.py:87-88
-    float mult = neg / pos;                                  // nmf.py:89
-    if (a.gamma != 1.0f) mult = powf(mult, a.gamma);         // nmf.py:90-91
-    newv = p * mult;                                         // nmf.py:92
+    newv = mu_step(p, num, pos, a.l1, a.l2, a.gamma);
     a.param[idx] = newv;
   }
   if (a.absmax_bits) {          // one atomic per block: tens of thousands of same-address atomics serialise in L2
@@ -195,13 +190,8 @@ apply_update_vec4_kernel(ApplyArgs a) {
     auto one = [&](float pv, float n, float d) {
       n *= sc;
       if (a.kappa) n = fmaf(*a.kappa, a.kappa_vec[r], n);
-      const float neg = fmaxf(n, 0.f) + kEps;                  // nmf.py:78
-      float pos = a.den ? fmaxf(d * sc, 0.f) + kEps : klden;   // nmf.py:83 / :368-369
-      if (a.l1 > 0.f) pos += a.l1;                             // nmf.py:85-86
-      if (a.l2 > 0.f) pos = fmaf(a.l2, pv, pos);               // nmf.py:87-88
-      float mult = neg / pos;                                  // nmf.py:89
-      if (a.gamma != 1.0f) mult = powf(mult, a.gamma);         // nmf.py:90-91
-      return pv * mult;                                        // nmf.py:92
+      const float pos = a.den ? fmaxf(d * sc, 0.f) + kEps : klden;   // nmf.py:83 / :368-369
+      return mu_step(pv, n, pos, a.l1, a.l2, a.gamma);
     };
     p.x = one(p.x, num.x, den.x); p.y = one(p.y, num.y, den.y); p.z = one(p.z, num.z, den.z); p.w = one(p.w, num.w, den.w);
     *reinterpret_cast<float4*>(a.param + idx) = p;

@@ -42,9 +42,6 @@ def _check_f32_cuda(t, name, device):
 # contexts.  release_workspaces() drops them all.
 _WORKSPACES = {}
 _MAX_WORKSPACES = 2
-# fit(): take every 10th iteration's loss out of the next W update's contraction pass where the library folds it
-# (nmfb200_nmf_loss_prefetch_w).  NMFB200_LOSS_FOLD=0: always the loss pass of its own (A/B timing).
-LOSS_FOLD = os.environ.get("NMFB200_LOSS_FOLD", "1") != "0"
 _CACHE_BYTES = int(float(os.environ.get("NMFB200_WORKSPACE_CACHE_MB", "8192")) * (1 << 20))
 
 
@@ -215,7 +212,7 @@ class CudaNmfEngine(_CudaEngine):
                                                    l2_reg, _stream(self.device)))
 
     def iterate(self, n_iter, beta, gamma, l1_reg, l2_reg):
-        """n_iter x (update_w; update_h) in one call (CUDA-graph replay on the tensor-core path)."""
+        """n_iter x (update_w; update_h) in one host call."""
         _capi.check(self._lib.nmfb200_nmf_iterate(self._ctx, _ptr(self.W), _ptr(self.H), beta, gamma, l1_reg, l2_reg,
                                                   int(n_iter), _stream(self.device)))
 

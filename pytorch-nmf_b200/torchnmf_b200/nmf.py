@@ -249,7 +249,7 @@ class BaseComponent(torch.nn.Module):
             def fit_loss(more=False):
                 # `more`: a W update follows on these very factors -- the engine may take the loss out of that update's own
                 # contraction pass (engine.loss_prefetch_w) instead of a pass over V of its own
-                fold = more and _engine.LOSS_FOLD and hasattr(eng, "loss_prefetch_w")
+                fold = more and hasattr(eng, "loss_prefetch_w")
                 d = eng.loss_prefetch_w(beta) if fold else eng.loss(beta)
                 return math.sqrt(2.0 * d) if d >= 0 else float("nan")                      # nmf.py:362,402
 

@@ -1,9 +1,7 @@
-"""Board power and SM clock while the fused contraction runs back to back for ~2 s per setting (tuning build, knock-out
-bits of tools/tc_knock.py).  Shows what the launch costs in a burst vs sustained, and which part of the kernel the
-power goes to (knocked-out results are numerically invalid)."""
+"""Board power and SM clock while the fused contraction runs back to back for ~2 s.  Shows what the launch costs in a
+burst vs sustained."""
 import os, sys, subprocess, statistics, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-os.environ.setdefault("NMFB200_LIB", os.path.join(ROOT, "pytorch-nmf_b200", "lib", "trace", "libnmf_b200.so"))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "pytorch-nmf_b200")]
 import torch
 from torchnmf_b200.engine import CudaNmfEngine, release_workspaces
@@ -12,32 +10,26 @@ N, C, R = 65536, 4096, 64
 torch.manual_seed(0)
 V = torch.rand(N, C, device="cuda").bfloat16().float()
 W = torch.randn(C, R, device="cuda").abs(); H = torch.randn(N, R, device="cuda").abs()
-ks = [int(x) for x in sys.argv[2].split(",")] if len(sys.argv) > 2 else [0, 4, 8, 16, 24, 32, 36, 56, 60]
-names = {0: "full kernel", 4: "ratio = TMEM ld/st only", 8: "no O-MMA", 16: "no S-MMA", 24: "no MMA", 32: "no V loads (no HBM stream)",
-         36: "no V loads, no ratio math", 56: "no MMA, no V loads", 60: "pipeline skeleton only"}
-for k in ks:
-    os.environ["NMFB200_TC_KNOCK"] = str(k)
-    eng = CudaNmfEngine(V, W, H, prec)
-    for _ in range(5): eng.contract_only(1, 1.0)
-    torch.cuda.synchronize()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    for _ in range(10): eng.contract_only(1, 1.0)
-    e1.record(); torch.cuda.synchronize()
-    burst = e0.elapsed_time(e1) / 10 * 1e3
-    time.sleep(1.0)
-    smi = subprocess.Popen(["nvidia-smi", "--query-gpu=power.draw,clocks.sm", "--format=csv,noheader,nounits", "-lms", "50"],
-                           stdout=subprocess.PIPE, text=True)
-    n = int(2.0e6 / burst)
-    e0.record()
-    for _ in range(n): eng.contract_only(1, 1.0)
-    e1.record(); torch.cuda.synchronize()
-    sus = e0.elapsed_time(e1) / n * 1e3
-    smi.terminate()
-    rows = [l.split(",") for l in smi.stdout.read().strip().splitlines() if "," in l]
-    pw = sorted(float(r[0]) for r in rows); ck = sorted(float(r[1]) for r in rows)
-    top = pw[len(pw) // 2:]                       # samples taken under load (the first ones still ramp)
-    print(f"knock {k:2d} {names.get(k, ''):32s} burst {burst:6.1f} us  sustained {sus:6.1f} us  power {statistics.median(top):5.0f} W  "
-          f"clock {statistics.median(ck[:len(ck) // 2 + 1]):5.0f} MHz ({len(rows)} samples)", flush=True)
-    eng.close(); release_workspaces()
-    time.sleep(1.0)
+eng = CudaNmfEngine(V, W, H, prec)
+for _ in range(5): eng.contract_only(1, 1.0)
+torch.cuda.synchronize()
+e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+e0.record()
+for _ in range(10): eng.contract_only(1, 1.0)
+e1.record(); torch.cuda.synchronize()
+burst = e0.elapsed_time(e1) / 10 * 1e3
+time.sleep(1.0)
+smi = subprocess.Popen(["nvidia-smi", "--query-gpu=power.draw,clocks.sm", "--format=csv,noheader,nounits", "-lms", "50"],
+                       stdout=subprocess.PIPE, text=True)
+n = int(2.0e6 / burst)
+e0.record()
+for _ in range(n): eng.contract_only(1, 1.0)
+e1.record(); torch.cuda.synchronize()
+sus = e0.elapsed_time(e1) / n * 1e3
+smi.terminate()
+rows = [l.split(",") for l in smi.stdout.read().strip().splitlines() if "," in l]
+pw = sorted(float(r[0]) for r in rows); ck = sorted(float(r[1]) for r in rows)
+top = pw[len(pw) // 2:]                       # samples taken under load (the first ones still ramp)
+print(f"full kernel  burst {burst:6.1f} us  sustained {sus:6.1f} us  power {statistics.median(top):5.0f} W  "
+      f"clock {statistics.median(ck[:len(ck) // 2 + 1]):5.0f} MHz ({len(rows)} samples)", flush=True)
+eng.close(); release_workspaces()

@@ -16,6 +16,6 @@ try:
         if i % 200 == 199:
             eng.check_health()
     eng.check_health()
-    print(f"OK   {prec} var={os.environ.get('NMFB200_TC_VARIANT')} N={N} C={C} {reps} launches {time.time()-t0:.2f}s", flush=True)
+    print(f"OK   {prec} N={N} C={C} {reps} launches {time.time()-t0:.2f}s", flush=True)
 except Exception as e:
-    print(f"FAIL {prec} var={os.environ.get('NMFB200_TC_VARIANT')} N={N} C={C} after {time.time()-t0:.3f}s: {str(e)[:80]}", flush=True)
+    print(f"FAIL {prec} N={N} C={C} after {time.time()-t0:.3f}s: {str(e)[:80]}", flush=True)
