@@ -126,6 +126,9 @@ bool use_tc(const nmfb200_ctx* c, double beta) {
   return c->tc != nullptr && !c->tc_off && tc_supports_beta(c->tc, beta);
 }
 
+// NMFD: beta = 1 on tensor cores (tc_nmfd.cu), everything else on the fp32 sliding GEMMs (nmfd.cu)
+bool nmfd_use_tc(const nmfb200_ctx* c, double beta) { return c->tcd && !c->tc_off && beta == 1.0; }
+
 }  // namespace
 
 extern "C" {
@@ -221,7 +224,7 @@ int nmfb200_precision(const nmfb200_ctx* ctx) {
 
 int nmfb200_precision_for_beta(const nmfb200_ctx* ctx, double beta) {
   if (!ctx) return -100;
-  if (ctx->kind == 1) return (ctx->tcd && !ctx->tc_off && tc_nmfd_supported(ctx->d, beta)) ? NMFB200_PREC_F16 : NMFB200_PREC_F32;
+  if (ctx->kind == 1) return nmfd_use_tc(ctx, beta) ? NMFB200_PREC_F16 : NMFB200_PREC_F32;
   if (ctx->kind != 0 || !use_tc(ctx, beta)) return NMFB200_PREC_F32;
   // beta != 1 kernels read only the hi halves of the operand copies
   return (beta == 1.0 || beta == 2.0) ? ctx->precision : NMFB200_PREC_F16;
@@ -595,14 +598,20 @@ static int nmfd_create_impl(nmfb200_ctx** out, int device, int64_t B, int64_t C,
   const bool one_d = X[0] == 1 && X[1] == 1;
   if (!one_d && precision == NMFB200_PREC_F16)
     return fail(NMFB200_ERR_INVALID, "NMF2D / NMF3D run on the fp32 kernels (precision auto or f32)");
+  NmfdShape d{(int)B, (int)C, (int)L, (int)R, (int)T, (int)(L - T + 1)};
+  d.X1 = (int)X[0]; d.X2 = (int)X[1]; d.T1 = (int)K[0]; d.T2 = (int)K[1];
+  // AUTO: the tensor-core kernels wherever they compute the shape (beta = 1 only: nmfd_use_tc); fp32 everywhere else
+  const bool tc_shape = tc_nmfd_shape_supported(d);
+  if (precision == NMFB200_PREC_F16 && !tc_shape)
+    return fail(NMFB200_ERR_INVALID, "shape not supported by the tensor-core NMFD path (need T <= 128)");
   DeviceGuard guard(device);
   if (!guard.ok) return fail(NMFB200_ERR_CUDA, "cannot select the requested device");
   nmfb200_ctx* c = new (std::nothrow) nmfb200_ctx();
   if (!c) return fail(NMFB200_ERR_INVALID, "out of host memory");
-  c->kind = 1; c->device = device; c->precision = precision == NMFB200_PREC_F32 ? NMFB200_PREC_F32 : NMFB200_PREC_F16; c->R = R;
+  c->kind = 1; c->device = device; c->R = R;
+  c->precision = (precision == NMFB200_PREC_F16 || (precision == NMFB200_PREC_AUTO && tc_shape)) ? NMFB200_PREC_F16 : NMFB200_PREC_F32;
   c->auto_mode = precision == NMFB200_PREC_AUTO;
-  c->d = NmfdShape{(int)B, (int)C, (int)L, (int)R, (int)T, (int)(L - T + 1)};
-  c->d.X1 = (int)X[0]; c->d.X2 = (int)X[1]; c->d.T1 = (int)K[0]; c->d.T2 = (int)K[1];
+  c->d = d;
   c->dgrad_nsplit = nmfd_dgrad_nsplit(c->d);
   c->wgrad_nsplit = nmfd_wgrad_nsplit(c->d);
   int64_t pf = (int64_t)c->wgrad_nsplit * C * R * c->d.w_inner();
@@ -623,7 +632,7 @@ static int nmfd_create_impl(nmfb200_ctx** out, int device, int64_t B, int64_t C,
     free_ctx(c);
     return fail(NMFB200_ERR_CUDA, std::string("cudaMalloc: ") + cudaGetErrorString(e));
   }
-  if (c->precision != NMFB200_PREC_F32 && one_d) {       // the tensor-core kernels cover the one-axis case
+  if (c->precision == NMFB200_PREC_F16) {
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, device) == cudaSuccess && prop.major == 10) {
       int rc = tc_nmfd_create(&c->tcd, c->d);          // beta = 1 runs as tcgen05 sliding GEMMs (tc_nmfd.cu)
@@ -672,14 +681,6 @@ int nmfb200_nmfd_set_target(nmfb200_ctx* ctx, const float* V, void* stream) {
   return 0;
 }
 
-// beta = 1 on tensor cores: both column-sum vectors (KL denominators, nmf.py:122-131, and kappa), then the recon pass
-static bool nmfd_use_tc(const nmfb200_ctx* c, double beta) {
-  return c->tcd != nullptr && !c->tc_off && tc_nmfd_supported(c->d, beta);
-}
-static int nmfd_tc_recon(nmfb200_ctx* c, const float* W, const float* H, bool loss, double* loss_dev, cudaStream_t st) {
-  return tc_nmfd_recon(c->tcd, c->V, W, H, loss, loss_dev, st);
-}
-
 static int nmfd_phi(nmfb200_ctx* c, const float* W, const float* H, double beta, cudaStream_t st) {
   if (beta != 1.0) {
     if (!c->Pp) NMF_CUDA_CHECK(cudaMalloc(&c->Pp, (size_t)c->d.B * c->d.C * c->d.v_inner() * sizeof(float)));
@@ -701,7 +702,7 @@ static int nmfd_terms(nmfb200_ctx* ctx, const float* W, const float* H, int whic
   a.chunk_stride = a.numel; a.ldp = a.rowlen; a.out_scale = nullptr; a.absmax_bits = nullptr;
   *tc = nmfd_use_tc(ctx, beta);
   if (*tc) {
-    int rc = nmfd_tc_recon(ctx, W, H, false, nullptr, st);
+    int rc = tc_nmfd_recon(ctx->tcd, ctx->V, W, H, false, nullptr, st);
     if (rc) return rc;
     const float* part; int nsplit;
     rc = which == 0 ? tc_nmfd_wgrad(ctx->tcd, &part, &nsplit, st) : tc_nmfd_dgrad(ctx->tcd, &part, &nsplit, st);
@@ -790,7 +791,7 @@ int nmfb200_nmfd_loss(nmfb200_ctx* ctx, const float* W, const float* H, double b
   CTX_GUARD(ctx, 1);
   if (!ctx->has_target) return fail(NMFB200_ERR_STATE, "set_target has not been called");
   if (!W || !H || !loss_dev) return fail(NMFB200_ERR_INVALID, "null pointer");
-  if (nmfd_use_tc(ctx, beta)) return nmfd_tc_recon(ctx, W, H, true, loss_dev, (cudaStream_t)stream);
+  if (nmfd_use_tc(ctx, beta)) return tc_nmfd_recon(ctx->tcd, ctx->V, W, H, true, loss_dev, (cudaStream_t)stream);
   return nmfd_recon_phi(ctx->d, ctx->V, W, H, beta, nullptr, nullptr, ctx->loss_blocks, ctx->loss_max_blocks,
                         loss_dev, (cudaStream_t)stream);
 }

@@ -1,9 +1,11 @@
 // Thin inline-PTX wrappers for the sm_100a features the fused kernels use:
-// mbarrier, TMA (cp.async.bulk.tensor), tcgen05.{alloc,mma,commit,ld,st,fence}, UMMA descriptors.
+// mbarrier, TMA (cp.async.bulk.tensor), tcgen05.{alloc,mma,commit,ld,st,fence}, UMMA descriptors; and the host helpers
+// that tc_nmf.cu and tc_nmfd.cu share (tensor maps, the wait-abort record).
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdio.h>
 
 namespace nmfb200 {
 namespace ptx {
@@ -67,7 +69,7 @@ __device__ __forceinline__ bool mbar_try_wait_parked(uint32_t bar, uint32_t pari
 }
 // Bounded wait: on a protocol bug (no progress for ~1 s) the first waiter records (block, thread, barrier, parity)
 // in g_wait_abort and every wait in the grid then falls through, so the kernel terminates instead of hanging
-// the GPU box; the host checks the record after the launch (tc_nmf.cu: check_wait_abort).
+// the GPU box; the host checks the record after the launch (check_wait_abort below).
 static __device__ unsigned int g_wait_abort[8];      // one record per translation unit (tc_nmf.cu, tc_nmfd.cu)
 // Slow path of mbar_wait, out of line on purpose: the warp-specialised loops are latency-bound serial instruction
 // streams (one MMA-issuing warp feeds the whole SM), so every wait site inlines only try_wait + a predicated call.
@@ -248,5 +250,23 @@ __device__ __forceinline__ uint32_t pack_f16x2_sat(float lo, float hi) {
   return d;
 }
 
+// ---- host side ------------------------------------------------------------------------------------------
+// After a stream synchronise: report (to stderr, after `label`) and clear the wait-abort record of the translation unit this
+// is compiled into.  1: one of its kernels aborted a wait since the last check; 0: none did; -1: the record is unreadable.
+static inline int check_wait_abort(const char* label) {
+  unsigned int h[8] = {0};
+  if (cudaMemcpyFromSymbol(h, g_wait_abort, sizeof(h)) != cudaSuccess) return -1;
+  if (!h[0]) return 0;
+  fprintf(stderr, "nmf_b200: %smbarrier wait aborted: block %u thread %u (warp %u) bar_addr %u parity %u\n", label, h[1], h[2],
+          h[2] / 32, h[3], h[4]);
+  const unsigned int z[8] = {0};
+  cudaMemcpyToSymbol(g_wait_abort, z, sizeof(z));
+  return 1;
+}
+
 }  // namespace ptx
+
+// 2-D fp16 row-major tensor map (rows x cols, row pitch ld elements), box 64 cols x box_rows rows, SWIZZLE_128B (tc_nmf.cu)
+int make_tmap(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows);
+
 }  // namespace nmfb200

@@ -1528,33 +1528,6 @@ sum_blocks_kernel(const double* __restrict__ blockpart, int n, double* __restric
 
 // ---- host side --------------------------------------------------------------------------------------
 
-PFN_cuTensorMapEncodeTiled_v12000 get_encode_fn() {
-  static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
-  if (fn) return fn;
-  void* ptr = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) != cudaSuccess ||
-      qres != cudaDriverEntryPointSuccess)
-    return nullptr;
-  fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(ptr);
-  return fn;
-}
-
-// 2-D fp16 row-major tensor (rows x cols, row pitch ld elements), box 64 cols x box_rows rows, SWIZZLE_128B
-int make_tmap(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
-  auto fn = get_encode_fn();
-  if (!fn) { set_error("cuTensorMapEncodeTiled entry point not available"); return 2; }
-  cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t gstr[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), gdim, gstr, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed with code " + std::to_string((int)r)); return 2; }
-  return 0;
-}
-
 struct Plan { int row_blocks, tiles, nchunks, tpc; };
 
 Plan make_plan(int64_t Mr, int64_t Nc, int num_sms, int TN) {
@@ -1580,6 +1553,32 @@ Plan make_plan(int64_t Mr, int64_t Nc, int num_sms, int TN) {
 }
 
 }  // namespace
+
+static PFN_cuTensorMapEncodeTiled_v12000 get_encode_fn() {
+  static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
+  if (fn) return fn;
+  void* ptr = nullptr;
+  cudaDriverEntryPointQueryResult qres;
+  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) != cudaSuccess ||
+      qres != cudaDriverEntryPointSuccess)
+    return nullptr;
+  fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(ptr);
+  return fn;
+}
+
+int make_tmap(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
+  auto fn = get_encode_fn();
+  if (!fn) { set_error("cuTensorMapEncodeTiled entry point not available"); return 2; }
+  cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+  cuuint64_t gstr[1] = {(cuuint64_t)ld * 2};
+  cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
+  cuuint32_t estr[2] = {1, 1};
+  CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), gdim, gstr, box, estr,
+                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed with code " + std::to_string((int)r)); return 2; }
+  return 0;
+}
 
 struct TcState {
   // ---- row-sharded W update over peer memory (tc_peer_*): one cudaMalloc block per rank, shared by CUDA IPC:
@@ -2149,17 +2148,8 @@ int tc_peer_check(TcState* s, cudaStream_t st) {
 
 // debugging aid: report (and clear) a recorded mbarrier wait abort; synchronises the stream
 int tc_check_wait_abort(cudaStream_t st) {
-  unsigned int h[8] = {0};
   if (cudaStreamSynchronize(st) != cudaSuccess) return -1;
-  cudaMemcpyFromSymbol(h, ptx::g_wait_abort, sizeof(h));
-  if (h[0]) {
-    fprintf(stderr, "nmf_b200: mbarrier wait aborted: block %u thread %u (warp %u) bar_addr %u parity %u\n", h[1], h[2], h[2] / 32,
-            h[3], h[4]);
-    unsigned int z[8] = {0};
-    cudaMemcpyToSymbol(ptx::g_wait_abort, z, sizeof(z));
-    return 1;
-  }
-  return 0;
+  return ptx::check_wait_abort("");
 }
 
 int tc_contract_only(TcState* s, const float* W, const float* H, int which, double beta, cudaStream_t st) {

@@ -5,13 +5,19 @@
 //   wgrad : gW[c, r, t] = sum_l  P~[c, l] H[r, l-t]              (W update: numerator = gW / 2^.. + kappa colsum(H))
 //   dgrad : gH[r, j]    = sum_{c,t} W[c,r,t] P~[c, j+t]          (H update: numerator = gH / 2^.. + kappa colsum(W))
 //
-// Each is a GEMM whose one operand is a plain matrix (TMA, SWIZZLE_128B) and whose other operand is a Toeplitz / Hankel
-// matrix: row i of a 128 x 64 tile is the 64-element window of ONE fp16 vector (a padded row of H, or a row of P~) that
-// starts one element further than row i - 1 (recon, dgrad) or one element earlier (wgrad).  Nothing of that matrix ever
-// exists in global memory: per k-block the TMA warp bulk-copies the ~200-element source window into shared memory and
-// the eight producer warps write the 128 x 64 tile from it in the UMMA SWIZZLE_128B K-major layout (4-byte shared loads,
-// one byte-permute per word for odd shifts, 16-byte stores), 2 threads per row.  The MMA warp issues tcgen05.mma SS on
-// it exactly as on a TMA-written tile; accumulators live in TMEM; the epilogue warps read them back with tcgen05.ld.
+// recon and dgrad use the eight-phase formulation (tcnmfd_recon2_kernel, tcnmfd_dgrad2_kernel): the big operand is the raw
+// fp16 row in shared memory under an overlapping descriptor, the small one eight shifted copies of W.  wgrad
+// (tcnmfd_wgrad_kernel) is a GEMM whose A operand is a plain matrix (P~, TMA, SWIZZLE_128B) and whose B operand is a
+// Toeplitz matrix: row t of a 128 x 64 tile is the 64-element window of a padded row of H that starts one element earlier
+// than row t - 1.  Nothing of that matrix ever exists in global memory: per k-block the TMA warp bulk-copies the
+// ~200-element source window into shared memory and the eight producer warps write the 128 x 64 tile from it in the UMMA
+// SWIZZLE_128B K-major layout (4-byte shared loads, one byte-permute per word for odd shifts, 16-byte stores), 2 threads
+// per row.  The MMA warp issues tcgen05.mma SS on it exactly as on a TMA-written tile; the accumulator lives in TMEM; the
+// epilogue warps read it back with tcgen05.ld.
+//
+// Scope: T <= 128 (tc_nmfd_shape_supported).  wgrad holds every shift of a (128-row c tile, component) in ONE 128 x 128
+// accumulator whose columns are the shifts, and at T = 128 the eight-phase stages take about 110 KB of shared memory.
+// Longer kernels run on the fp32 sliding GEMMs of nmfd.cu.
 //
 // Precision design = the NMF kernel's (DESIGN.md 4.2): fp16 operands with power-of-two scales, fp32 accumulation, the
 // ratio tile centred on kappa = sum(V) / sum(WH) so that the K = 8192 ... 131200-term numerator sums are signed and small
@@ -19,10 +25,8 @@
 #include "tc_nmfd.cuh"
 
 #include <cuda.h>
-#include <cudaTypedefs.h>
 
 #include <algorithm>
-#include <cstdlib>
 #include <string>
 
 #include "sm100_ptx.cuh"
@@ -37,22 +41,14 @@ constexpr int kStages = 3;
 constexpr int kWinHalfs = 256;     // source window per k-block: 128 rows + 64 columns + alignment slack (512 bytes)
 constexpr int kThreads = 384;      // warp 0 TMA | warp 1 MMA | warps 2-3 idle | warps 4-11 producers (8-11 also epilogue)
 
-enum : int { kRecon = 0, kReconLoss = 1, kWgrad = 2, kDgrad = 3 };
-
-struct NmfdTcParams {
-  int B, C, L, R, T, Lin, Tp;     // Tp = T rounded up to 64
+struct WgradParams {
+  int B, C, L, R, T;
   int Lp;                         // padded row length of Hp16 (halfs); H[b,r,j] sits at column padl + j
   int padl;
-  int Lq;                         // row pitch of P16 (halfs), >= L + 72, zero beyond L
   const __half* Hp16;             // [B*R][Lp]
-  const __half* P16;              // [B*C][Lq]      (wgrad / dgrad source)
-  __half* P16out;                 // recon output
-  const float* V;                 // [B][C][L] fp32
   const int* exps;                // {eW, eH, eP}: power-of-two exponents of W16, Hp16, P16
-  const float* kappa;             // device scalar
-  float* out;                     // wgrad: [nsplit][C][R][T]   dgrad: [nsplit][B][R][Lin]
-  double* loss_part;              // recon loss: one partial per CTA
-  int nsplit, kb_per_split;
+  float* out;                     // [nsplit][C][R][T]
+  int kb_per_split;
 };
 
 struct Smem {
@@ -63,8 +59,7 @@ struct Smem {
   static constexpr int kBar = kWin + kStages * kWinHalfs * 2;
   static constexpr int kNumBars = 4 * kStages + 1;           // win_full, tile_full, empty, win_read per stage + acc_full
   static constexpr int kTmemPtr = kBar + 8 * kNumBars;
-  static constexpr int kRed = kTmemPtr + 16;
-  static constexpr int kTotal = kRed + 8 * 16;
+  static constexpr int kTotal = kTmemPtr + 16;
 };
 
 __device__ __forceinline__ void bulk_copy_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
@@ -73,13 +68,10 @@ __device__ __forceinline__ void bulk_copy_g2s(uint32_t dst, const void* src, uin
                : "memory");
 }
 
-// One kernel, four roles of the same pipeline (KIND):
-//   recon / recon-loss : grid (L tiles, C tiles, B);  plain = A = Wr16 tile (rows c), Toeplitz = B (rows l), N = 128
-//   wgrad              : grid (C tiles, R, nsplit);   plain = A = P16 tile (rows c),  Toeplitz = B (rows t), N = 128
-//   dgrad              : grid (Lin tiles, nsplit, B); Toeplitz = A (rows j), plain = B = Wf16 rows (c R + r), N = Rp16
-template <int KIND>
+// grid (C tiles, R, nsplit): A = P16 tile (rows c, by TMA), B = Toeplitz tile of the H row of component blockIdx.y (rows t,
+// built by the producers), N = 128 shifts; split z walks k-blocks [kb_per_split z, kb_per_split (z + 1)) of (b, l)
 __global__ void __launch_bounds__(kThreads, 2)
-tcnmfd_kernel(const __grid_constant__ CUtensorMap tmPlain, const NmfdTcParams p) {
+tcnmfd_wgrad_kernel(const __grid_constant__ CUtensorMap tmP, const WgradParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t raw32 = ptx::smem_u32(smem_raw);
   const uint32_t sbase = (raw32 + 1023u) & ~1023u;
@@ -88,12 +80,9 @@ tcnmfd_kernel(const __grid_constant__ CUtensorMap tmPlain, const NmfdTcParams p)
   auto BAR = [&](int i) { return sbase + Smem::kBar + 8u * i; };
   constexpr int B_WIN = 0, B_TILE = kStages, B_EMPTY = 2 * kStages, B_WREAD = 3 * kStages, B_ACC = 4 * kStages;
   volatile uint32_t* tmem_ptr_smem = reinterpret_cast<volatile uint32_t*>(smem_al + Smem::kTmemPtr);
-  constexpr bool RECON = KIND == kRecon || KIND == kReconLoss;
-  const int Rp16 = (p.R + 15) & ~15;
-  const uint32_t ncols = KIND == kDgrad ? (Rp16 <= 32 ? 32u : (Rp16 <= 64 ? 64u : (Rp16 <= 128 ? 128u : 256u))) : 128u;
 
   if (warp == 0 && lane == 0) {
-    ptx::prefetch_tmap(&tmPlain);
+    ptx::prefetch_tmap(&tmP);
     for (int i = 0; i < kStages; ++i) {
       ptx::mbar_init(BAR(B_WIN + i), 1);
       ptx::mbar_init(BAR(B_TILE + i), 8);        // one arrival per producer warp
@@ -105,7 +94,7 @@ tcnmfd_kernel(const __grid_constant__ CUtensorMap tmPlain, const NmfdTcParams p)
     ptx::fence_proxy_async();
   }
   if (warp == 1) {
-    ptx::tmem_alloc(sbase + Smem::kTmemPtr, ncols);
+    ptx::tmem_alloc(sbase + Smem::kTmemPtr, 128);
     ptx::tmem_relinquish();
   }
   ptx::tc_fence_before();
@@ -113,40 +102,23 @@ tcnmfd_kernel(const __grid_constant__ CUtensorMap tmPlain, const NmfdTcParams p)
   ptx::tc_fence_after();
   const uint32_t tmem = *tmem_ptr_smem;
 
-  // ---- what this CTA computes, as a list of k-blocks: (plain-tile coordinates, source vector, window start) -------------
-  int nkb, kb0 = 0;
-  if (RECON) nkb = p.R * (p.Tp / kKB);
-  else { kb0 = (KIND == kWgrad ? blockIdx.z : blockIdx.y) * p.kb_per_split; nkb = p.kb_per_split; }
-  const int lkb = (p.L + kKB - 1) / kKB;                    // wgrad: k-blocks per batch element
-  const int tkb = p.Tp / kKB;
-  if (KIND == kWgrad) nkb = max(0, min(nkb, p.B * lkb - kb0));
-  if (KIND == kDgrad) nkb = max(0, min(nkb, p.C * tkb - kb0));
-  // per k-block: returns the plain tile's TMA coordinates (x = column, y = row), the source row pointer and the index of the
-  // source element that row 0 / column 0 of the Toeplitz tile reads; `dir` is the step of that index from row to row
+  // ---- what this CTA computes, as a list of k-blocks: (P16 tile coordinates, H row, window start) ------------------------
+  const int kb0 = blockIdx.z * p.kb_per_split;
+  const int lkb = (p.L + kKB - 1) / kKB;                    // k-blocks per batch element
+  const int nkb = max(0, min(p.kb_per_split, p.B * lkb - kb0));
+  // per k-block: returns the P16 tile's TMA coordinates (x = column, y = row), the H row pointer and the index of the H
+  // element that row 0 / column 0 of the Toeplitz tile reads; row t reads one element earlier than row t - 1
   auto kblock = [&](int kb, int& px, int& py, const __half*& src, int& e0) {
-    if (RECON) {
-      const int r = kb / tkb, kk = kb - r * tkb;            // k = reversed shift t' in [64 kk, 64 kk + 64)
-      px = r * p.Tp + kk * kKB; py = blockIdx.y * kM;
-      src = p.Hp16 + ((int64_t)blockIdx.z * p.R + r) * p.Lp;
-      e0 = p.padl + blockIdx.x * kM - p.Tp + 1 + kk * kKB;  // H index l - t = l - (Tp - 1 - t')
-    } else if (KIND == kWgrad) {
-      const int g = kb0 + kb, b = g / lkb, lk = g - b * lkb;
-      px = lk * kKB; py = b * p.C + blockIdx.x * kM;
-      src = p.Hp16 + ((int64_t)b * p.R + blockIdx.y) * p.Lp;
-      e0 = p.padl + lk * kKB;                               // row t reads H[l - t]: e0 - t
-    } else {
-      const int g = kb0 + kb, c = g / tkb, kk = g - c * tkb;
-      px = kk * kKB; py = c * p.R;
-      src = p.P16 + ((int64_t)blockIdx.z * p.C + c) * p.Lq;
-      e0 = blockIdx.x * kM + kk * kKB;                      // row j reads P[j + t]
-    }
+    const int g = kb0 + kb, b = g / lkb, lk = g - b * lkb;
+    px = lk * kKB; py = b * p.C + blockIdx.x * kM;
+    src = p.Hp16 + ((int64_t)b * p.R + blockIdx.y) * p.Lp;
+    e0 = p.padl + lk * kKB;                                 // row t reads H[l - t]: e0 - t
   };
-  constexpr int dir = KIND == kWgrad ? -1 : 1;
   // window = source elements [wbeg, wbeg + kWinHalfs), wbeg 8-aligned and <= the smallest index any row reads
-  auto win_begin = [&](int e0) { return (dir > 0 ? e0 : e0 - (kM - 1)) & ~7; };
+  auto win_begin = [&](int e0) { return (e0 - (kM - 1)) & ~7; };
 
   if (warp == 0) {
-    // =========================== TMA: plain operand tile + source window per k-block ==============================
+    // =========================== TMA: P16 tile + source window per k-block ===========================================
     if (lane == 0) {
       for (int kb = 0; kb < nkb; ++kb) {
         const int s = kb % kStages, ph = (kb / kStages) & 1;
@@ -154,31 +126,28 @@ tcnmfd_kernel(const __grid_constant__ CUtensorMap tmPlain, const NmfdTcParams p)
         ptx::mbar_wait(BAR(B_WREAD + s), ph ^ 1);      // ... and every producer warp has read its source window
         int px, py, e0; const __half* src;
         kblock(kb, px, py, src, e0);
-        const uint32_t plain_bytes = KIND == kDgrad ? (uint32_t)Rp16 * kKB * 2 : (uint32_t)Smem::kTile;
-        ptx::mbar_expect_tx(BAR(B_WIN + s), plain_bytes + kWinHalfs * 2);
-        ptx::tma_load_2d(&tmPlain, BAR(B_WIN + s), sbase + Smem::kPlain + s * Smem::kTile, px, py);
+        ptx::mbar_expect_tx(BAR(B_WIN + s), (uint32_t)Smem::kTile + kWinHalfs * 2);
+        ptx::tma_load_2d(&tmP, BAR(B_WIN + s), sbase + Smem::kPlain + s * Smem::kTile, px, py);
         bulk_copy_g2s(sbase + Smem::kWin + s * kWinHalfs * 2, src + win_begin(e0), kWinHalfs * 2, BAR(B_WIN + s));
       }
     }
   } else if (warp == 1) {
     // =========================== MMA issuer ==========================================================================
-    const uint32_t nmma = KIND == kDgrad ? (uint32_t)Rp16 : 128u;
-    const uint32_t idesc = ptx::idesc_f16(kM, (int)nmma, 0, 0);
+    const uint32_t idesc = ptx::idesc_f16(kM, 128, 0, 0);
     constexpr uint32_t descHi = ptx::smem_desc_hi_sw128(1024);
     for (int kb = 0; kb < nkb; ++kb) {
       const int s = kb % kStages, ph = (kb / kStages) & 1;
       if (lane == 0) {
-        ptx::mbar_wait(BAR(B_WIN + s), ph);       // plain tile landed (TMA -> this thread)
+        ptx::mbar_wait(BAR(B_WIN + s), ph);       // P16 tile landed (TMA -> this thread)
         ptx::mbar_wait(BAR(B_TILE + s), ph);      // Toeplitz tile written by the 8 producer warps
       }
       __syncwarp();
       ptx::tc_fence_after();
       const uint32_t plain = sbase + Smem::kPlain + s * Smem::kTile, toep = sbase + Smem::kToep + s * Smem::kTile;
-      const uint32_t aBase = KIND == kDgrad ? toep : plain, bBase = KIND == kDgrad ? plain : toep;
       if (ptx::elect_one()) {
 #pragma unroll
         for (int ks = 0; ks < kKB / 16; ++ks) {
-          const uint32_t alo = ptx::smem_desc_lo(aBase, 16) + 2 * ks, blo = ptx::smem_desc_lo(bBase, 16) + 2 * ks;
+          const uint32_t alo = ptx::smem_desc_lo(plain, 16) + 2 * ks, blo = ptx::smem_desc_lo(toep, 16) + 2 * ks;
           ptx::mma_ss(tmem, ptx::make_desc(alo, descHi), ptx::make_desc(blo, descHi), idesc, (kb | ks) ? 1u : 0u);
         }
         ptx::mma_commit(BAR(B_EMPTY + s));
@@ -194,8 +163,8 @@ tcnmfd_kernel(const __grid_constant__ CUtensorMap tmPlain, const NmfdTcParams p)
       const int s = kb % kStages, ph = (kb / kStages) & 1;
       int px, py, e0; const __half* src;
       kblock(kb, px, py, src, e0);
-      const int off = e0 + dir * row - win_begin(e0) + 32 * half;        // first window element this thread reads (>= 0)
-      ptx::mbar_wait(BAR(B_WIN + s), ph);                               // window (and plain tile) landed
+      const int off = e0 - row - win_begin(e0) + 32 * half;             // first window element this thread reads (>= 0)
+      ptx::mbar_wait(BAR(B_WIN + s), ph);                               // window (and P16 tile) landed
       const uint32_t win = sbase + Smem::kWin + s * kWinHalfs * 2 + (uint32_t)(off >> 1) * 4;
       uint32_t w[17];
 #pragma unroll
@@ -217,93 +186,30 @@ tcnmfd_kernel(const __grid_constant__ CUtensorMap tmPlain, const NmfdTcParams p)
       if (lane == 0) { ptx::mbar_arrive(BAR(B_TILE + s)); ptx::mbar_arrive(BAR(B_WREAD + s)); }
     }
     if (warp >= 8) {
-      // =========================== epilogue (warps 8-11 = TMEM lane quarters 0-3) =====================================
+      // =========================== epilogue (warps 8-11 = TMEM lane quarters 0-3): row c, columns t ==================
       const int q = warp & 3, r128 = q * 32 + lane;
       const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
       ptx::mbar_wait(BAR(B_ACC), 0);
       ptx::tc_fence_after();
-      const float sc = exp2f(-(float)(p.exps[KIND == kDgrad ? 0 : (RECON ? 0 : 2)] + p.exps[RECON ? 1 : (KIND == kWgrad ? 1 : 2)]));
-      if (RECON) {
-        const int c = blockIdx.y * kM + r128, b = blockIdx.z, l0 = blockIdx.x * kM;
-        const bool row_ok = c < p.C;
-        const float kap = *p.kappa, pscale = exp2f((float)p.exps[2]);
-        const float* vrow = p.V + ((int64_t)b * p.C + (row_ok ? c : 0)) * p.L;
-        __half* prow = p.P16out + ((int64_t)b * p.C + (row_ok ? c : 0)) * p.Lq;
-        double acc = 0.0;
+      const float sc = exp2f(-(float)(p.exps[2] + p.exps[1]));
+      const int c = blockIdx.x * kM + r128, r = blockIdx.y;
+      float* dst = p.out + (((int64_t)blockIdx.z * p.C + (c < p.C ? c : 0)) * p.R + r) * p.T;    // [split][C][R][T]
+      const bool vec = (p.T & 3) == 0;
 #pragma unroll 1
-        for (int j = 0; j < kM / 16; ++j) {
-          uint32_t sr[16];
-          ptx::tmem_ld16(tmem + lane_addr + j * 16, sr);
-          ptx::tc_wait_ld();
-          const int l = l0 + j * 16;
-          float v[16];
+      for (int j = 0; j < kM / 16; ++j) {
+        uint32_t sr[16];
+        ptx::tmem_ld16(tmem + lane_addr + j * 16, sr);
+        ptx::tc_wait_ld();
+        if (c < p.C && j * 16 < p.T) {
+          if (vec && j * 16 + 16 <= p.T) {
 #pragma unroll
-          for (int i = 0; i < 16; ++i) v[i] = (row_ok && l + i < p.L) ? vrow[l + i] : 0.f;
-          if (KIND == kReconLoss) {
-            float a = 0.f;
-#pragma unroll
-            for (int i = 0; i < 16; ++i) {
-              const float x = __uint_as_float(sr[i]) * sc;
-              if (row_ok && l + i < p.L) a += v[i] * (logf(v[i] + kEps) - logf(x + kEps)) - v[i] + x;     // metrics.py:22
-            }
-            acc += (double)a;
+            for (int i = 0; i < 16; i += 4)
+              *reinterpret_cast<float4*>(dst + j * 16 + i) = make_float4(__uint_as_float(sr[i]) * sc, __uint_as_float(sr[i + 1]) * sc,
+                                                                         __uint_as_float(sr[i + 2]) * sc, __uint_as_float(sr[i + 3]) * sc);
           } else {
-            uint32_t pk[8];
 #pragma unroll
-            for (int i = 0; i < 8; ++i) {
-              const float x0 = fmaf(__uint_as_float(sr[2 * i]), sc, kEps), x1 = fmaf(__uint_as_float(sr[2 * i + 1]), sc, kEps);
-              const float p0 = (v[2 * i] / x0 - kap) * pscale, p1 = (v[2 * i + 1] / x1 - kap) * pscale;      // nmf.py:65, centred
-              pk[i] = ptx::pack_f16x2_sat((l + 2 * i < p.L) ? p0 : 0.f, (l + 2 * i + 1 < p.L) ? p1 : 0.f);
-            }
-            if (row_ok && l < p.Lq) {
-              *reinterpret_cast<uint4*>(prow + l) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-              *reinterpret_cast<uint4*>(prow + l + 8) = make_uint4(pk[4], pk[5], pk[6], pk[7]);
-            }
-          }
-        }
-        if (KIND == kReconLoss) {
-          double* red = reinterpret_cast<double*>(smem_al + Smem::kRed);
-          for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-          if (lane == 0) red[q] = acc;
-          asm volatile("bar.sync 1, 128;");
-          if (q == 0 && lane == 0)
-            p.loss_part[((int64_t)blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x] = (red[0] + red[1]) + (red[2] + red[3]);
-        }
-      } else if (KIND == kWgrad) {
-        const int c = blockIdx.x * kM + r128, r = blockIdx.y;
-        float* dst = p.out + (((int64_t)blockIdx.z * p.C + (c < p.C ? c : 0)) * p.R + r) * p.T;    // [split][C][R][T]
-        const bool vec = (p.T & 3) == 0;
-#pragma unroll 1
-        for (int j = 0; j < kM / 16; ++j) {
-          uint32_t sr[16];
-          ptx::tmem_ld16(tmem + lane_addr + j * 16, sr);
-          ptx::tc_wait_ld();
-          if (c < p.C && j * 16 < p.T) {
-            if (vec && j * 16 + 16 <= p.T) {
-#pragma unroll
-              for (int i = 0; i < 16; i += 4)
-                *reinterpret_cast<float4*>(dst + j * 16 + i) = make_float4(__uint_as_float(sr[i]) * sc, __uint_as_float(sr[i + 1]) * sc,
-                                                                           __uint_as_float(sr[i + 2]) * sc, __uint_as_float(sr[i + 3]) * sc);
-            } else {
-#pragma unroll
-              for (int i = 0; i < 16; ++i)
-                if (j * 16 + i < p.T) dst[j * 16 + i] = __uint_as_float(sr[i]) * sc;
-            }
-          }
-        }
-      } else {
-        const int j = blockIdx.x * kM + r128, b = blockIdx.z;
-#pragma unroll 1
-        for (int jj = 0; jj < Rp16 / 16; ++jj) {
-          uint32_t sr[16];
-          ptx::tmem_ld16(tmem + lane_addr + jj * 16, sr);
-          ptx::tc_wait_ld();
-          if (j < p.Lin) {
-#pragma unroll
-            for (int i = 0; i < 16; ++i) {
-              const int r = jj * 16 + i;
-              if (r < p.R) p.out[(((int64_t)blockIdx.y * p.B + b) * p.R + r) * p.Lin + j] = __uint_as_float(sr[i]) * sc;
-            }
+            for (int i = 0; i < 16; ++i)
+              if (j * 16 + i < p.T) dst[j * 16 + i] = __uint_as_float(sr[i]) * sc;
           }
         }
       }
@@ -311,7 +217,7 @@ tcnmfd_kernel(const __grid_constant__ CUtensorMap tmPlain, const NmfdTcParams p)
   }
   ptx::tc_fence_before();
   __syncthreads();
-  if (warp == 1) ptx::tmem_dealloc(tmem, ncols);
+  if (warp == 1) ptx::tmem_dealloc(tmem, 128);
 }
 
 // ---- dgrad, second formulation: no Toeplitz tile is built at all ---------------------------------------------------------
@@ -662,10 +568,8 @@ fold_colsum_kernel(const FoldTail f) {
   }
 }
 
-// One pass over W (C, R, T), block c: every fp16 operand copy of this row, scaled by 2^eW (eW from the max of W), written
+// One pass over W (C, R, T), block c: both fp16 operand copies of this row, scaled by 2^eW (eW from the max of W), written
 // 16 bytes per thread and step, plus the row's per-component sums (-> colsum_W, nmf.py:128-131):
-//   Wr16[c][r Tp + tt]           = W[c, r, Tp - 1 - tt]        (recon: shifts reversed so that the H window ascends)
-//   Wf16[c][r Tp + tt]           = W[c, r, tt]                 (dgrad, Toeplitz-tile formulation)
 //   Ws16[(c, grp, r%16, s)][u]   = W[c, r, u - s]              (dgrad, eight shifted copies)
 //   Wsh16[(c, s)][r Tq + u]      = W[c, r, s + A8 - u]         (recon, eight shifted copies)
 //
@@ -725,10 +629,9 @@ __device__ __forceinline__ void prep_w_shifted(const float* __restrict__ stage, 
 }
 
 __global__ void __launch_bounds__(256, 8)     // 8 blocks per SM: the 1025 blocks of cfg3 run as one wave
-prep_w_kernel(const float* __restrict__ W, int C, int R, int T, int Tp, int Tq, int ngroups,
-              const unsigned int* __restrict__ absmax, int* __restrict__ exps, __half* __restrict__ Wr16,
-              __half* __restrict__ Wf16, __half* __restrict__ Ws16, __half* __restrict__ Wsh16, int A8,
-              float* __restrict__ cs_part, int use_smem, int S, int F) {
+prep_w_kernel(const float* __restrict__ W, int C, int R, int T, int Tq, int ngroups,
+              const unsigned int* __restrict__ absmax, int* __restrict__ exps, __half* __restrict__ Ws16,
+              __half* __restrict__ Wsh16, int A8, float* __restrict__ cs_part, int use_smem, int S, int F) {
   const int e = pow2_exp14(__uint_as_float(*absmax));
   if (blockIdx.x == 0 && threadIdx.x == 0) exps[0] = e;
   const float sc = exp2f((float)e);
@@ -742,16 +645,6 @@ prep_w_kernel(const float* __restrict__ W, int C, int R, int T, int Tp, int Tq, 
     for (int i = 0; i < 4; ++i) h[i] = __floats2half2_rn(v[2 * i], v[2 * i + 1]);
     return *reinterpret_cast<const uint4*>(h);
   };
-  // plain forward / reversed copies: only read by the Toeplitz-tile kernels (A/B switches, very long shifts)
-  const int64_t rowlen = (int64_t)R * Tp;
-  for (int i8 = threadIdx.x; Wr16 != nullptr && i8 < R * Tp / 8; i8 += 256) {
-    const int i = i8 * 8, r = i / Tp, tt = i - r * Tp;
-    float f[8], rv[8];
-#pragma unroll
-    for (int k = 0; k < 8; ++k) { f[k] = w_at(r, tt + k); rv[k] = w_at(r, Tp - 1 - tt - k); }
-    *reinterpret_cast<uint4*>(Wf16 + c * rowlen + i) = pack8(f);
-    *reinterpret_cast<uint4*>(Wr16 + c * rowlen + i) = pack8(rv);
-  }
   if (use_smem) {
     for (int i = threadIdx.x; i < R * 8 * S; i += 256) stage[i] = 0.f;
     __syncthreads();
@@ -844,29 +737,34 @@ vsum_kernel(const float* __restrict__ V, int64_t n, double* __restrict__ part) {
   if (threadIdx.x == 0) { double t = 0.0; for (int i = 0; i < 8; ++i) t += sh[i]; part[blockIdx.x] = t; }
 }
 
-PFN_cuTensorMapEncodeTiled_v12000 encode_fn() {
-  static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
-  if (fn) return fn;
-  void* ptr = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) != cudaSuccess ||
-      qres != cudaDriverEntryPointSuccess)
-    return nullptr;
-  fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(ptr);
-  return fn;
+// Dynamic shared memory of each launch (bytes; the tcgen05 kernels' counts include 1 KB for aligning their base to 1024).
+// The recon2 / dgrad2 stages are the layouts computed at the top of those kernels; prep_w_kernel stages a row of W when it
+// fits (its division by multiplication also needs R T < 2^16) and reads it from global memory otherwise (0 bytes).
+struct KernelSmem {
+  int recon2, dgrad2, wgrad, prep_w;
+};
+
+KernelSmem kernel_smem(const NmfdShape& d, int Tq, int S) {
+  KernelSmem k;
+  const int nkk = Tq / kKB;
+  const uint32_t st_r = (((uint32_t)nkk * Smem::kTile + (uint32_t)(8 * kR2N + Tq) * 2) + 1023u) & ~1023u;
+  k.recon2 = (int)(kD2Stages * st_r + 8 * (2 * kD2Stages + 1) + 16 + 64 + 1024);
+  const uint32_t seg_pitch = (((uint32_t)(1024 + Tq) * 2) + 127u) & ~127u;
+  const uint32_t st_d = (((uint32_t)nkk * Smem::kTile + kD2Q * seg_pitch) + 1023u) & ~1023u;
+  k.dgrad2 = (int)(kD2Stages * st_d + 8 * (2 * kD2Stages + 1) + 16 + 1024);
+  k.wgrad = Smem::kTotal + 1024;
+  const size_t wrow_bytes = (size_t)d.R * 8 * S * sizeof(float);
+  k.prep_w = (wrow_bytes <= 200 * 1024 && (int64_t)d.R * d.T < 65536) ? (int)wrow_bytes : 0;
+  return k;
 }
 
-int make_tmap2(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
-  auto fn = encode_fn();
-  if (!fn) { set_error("cuTensorMapEncodeTiled entry point not available"); return 2; }
-  cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t gstr[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), gdim, gstr, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled (nmfd) failed with code " + std::to_string((int)r)); return 2; }
+// The limit is per kernel and per device, and other contexts on this device may need more than this one: only raise it.
+template <class Kernel>
+int raise_smem_limit(Kernel* kern, int bytes) {
+  cudaFuncAttributes fa;
+  NMF_CUDA_CHECK(cudaFuncGetAttributes(&fa, kern));
+  if (fa.maxDynamicSharedSizeBytes < bytes)
+    NMF_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
   return 0;
 }
 
@@ -874,16 +772,18 @@ int make_tmap2(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int
 
 struct TcNmfdState {
   NmfdShape d{};
-  int Tp = 0, Lp = 0, padl = 0, Lq = 0, Cpad = 0;
-  __half *Wr16 = nullptr, *Wf16 = nullptr, *Hp16 = nullptr, *P16 = nullptr, *Ws16 = nullptr, *Wsh16 = nullptr;
+  int Lp = 0, padl = 0, Lq = 0, Cpad = 0;
+  __half *Hp16 = nullptr, *P16 = nullptr, *Ws16 = nullptr, *Wsh16 = nullptr;
   int A8 = 0;                       // T - 1 rounded up to 8: alignment of the H window of the eight-phase recon
   int Tq = 0, ngroups = 1, cps_h2 = 0, ws_h2 = 1;   // dgrad2: padded shift extent, 16-component groups, c per split, splits
+  int ws_w = 1, kbs_w = 0;          // wgrad: splits, k-blocks per split
+  int prep_S = 0, prep_F = 0;       // staging layout of prep_w_kernel: S slots per shift-residue class, F leading zeros
+  KernelSmem smem{};
   float* part = nullptr;            // wgrad / dgrad split partials
   int64_t part_floats = 0;
   unsigned int* absmax = nullptr;   // [2]: max of W, max of H (float bits; written by absmax_kernel or by the ratio stage)
   float* colsum = nullptr;          // [2][R]: colsum_W | colsum_H
   float* cs_part = nullptr;         // per-row / per-block partial sums of the factor being refreshed
-  bool need_tile_copies = false;    // Wr16 / Wf16 are in use (see refresh)
   bool w_fresh = false, h_fresh = false;      // the fp16 copies / column sums of W, H match the fp32 factor
   bool aw_valid = false, ah_valid = false;    // absmax[0], absmax[1] hold the max of the current W, H
   int* exps = nullptr;              // {eW, eH, eP}
@@ -891,20 +791,17 @@ struct TcNmfdState {
   double* vsum = nullptr;           // [1] + [256] partials
   double* loss_part = nullptr;
   int loss_blocks = 0;
-  int ws_w = 1, ws_h = 1;           // split counts of wgrad / dgrad
-  int kbs_w = 0, kbs_h = 0;
-  CUtensorMap tmWr, tmWf, tmP, tmWs, tmWsh;
-  bool attr_set = false;
+  CUtensorMap tmP, tmWs, tmWsh;
 };
 
-bool tc_nmfd_supported(const NmfdShape& d, double beta) {
-  return beta == 1.0 && d.R >= 1 && d.R <= 256 && d.T >= 1 && d.L >= d.T;
+bool tc_nmfd_shape_supported(const NmfdShape& d) {
+  return d.one_d() && d.T >= 1 && d.T <= 128 && d.R >= 1 && d.R <= 256;
 }
 
 void tc_nmfd_destroy(TcNmfdState* s) {
   if (!s) return;
-  cudaFree(s->Wsh16); cudaFree(s->Ws16); cudaFree(s->Wr16); cudaFree(s->Wf16); cudaFree(s->Hp16); cudaFree(s->P16); cudaFree(s->part); cudaFree(s->absmax); cudaFree(s->colsum); cudaFree(s->cs_part);
-  cudaFree(s->exps); cudaFree(s->kappa); cudaFree(s->vsum); cudaFree(s->loss_part);
+  cudaFree(s->Wsh16); cudaFree(s->Ws16); cudaFree(s->Hp16); cudaFree(s->P16); cudaFree(s->part); cudaFree(s->absmax);
+  cudaFree(s->colsum); cudaFree(s->cs_part); cudaFree(s->exps); cudaFree(s->kappa); cudaFree(s->vsum); cudaFree(s->loss_part);
   delete s;
 }
 
@@ -912,37 +809,47 @@ int tc_nmfd_create(TcNmfdState** out, const NmfdShape& d) {
   *out = nullptr;
   TcNmfdState* s = new TcNmfdState();
   s->d = d;
-  s->Tp = (int)round_up(d.T, kKB);
-  s->padl = (int)round_up(s->Tp + 136, 8);                       // every window start >= 0 (padl >= A8 as well)
+  const int Tp = (int)round_up(d.T, kKB);
+  s->padl = (int)round_up(Tp + 136, 8);                          // every window start >= 0 (padl >= A8 as well)
   s->Lp = (int)round_up((int64_t)s->padl + round_up((int64_t)d.L, 8 * kR2N) + 256 + kWinHalfs + 136, 8);
   s->A8 = (int)round_up(d.T - 1, 8);
   s->Tq = (int)round_up(s->A8 + 8, kKB);                            // shifts u in [0, A8 + 7]; also covers dgrad's [0, T + 6]
   s->ngroups = (int)ceil_div(d.R, 16);
   s->Lq = (int)round_up(round_up((int64_t)d.L, 2048) + 1024 + s->Tq + kWinHalfs + 8, 8);
   s->Cpad = (int)round_up(d.C, kM);
-  const int lkb = (int)ceil_div(d.L, kKB), tkb = s->Tp / kKB;
   // split the K loops of wgrad / dgrad so that the grid is a few waves of 148 CTAs
-  const int64_t tiles_w = ceil_div(d.C, kM) * d.R, tiles_h = ceil_div(d.Lin, kM) * d.B;
-  int64_t kb_w = (int64_t)d.B * lkb, kb_h = (int64_t)d.C * tkb;
+  const int64_t tiles_w = ceil_div(d.C, kM) * d.R, kb_w = (int64_t)d.B * ceil_div(d.L, kKB);
   s->ws_w = (int)std::max<int64_t>(1, std::min<int64_t>(kb_w / 8, ceil_div(148 * 4, tiles_w)));
-  s->ws_h = (int)std::max<int64_t>(1, std::min<int64_t>(kb_h / 8, ceil_div(148 * 4, tiles_h)));
   s->kbs_w = (int)ceil_div(kb_w, s->ws_w); s->ws_w = (int)ceil_div(kb_w, s->kbs_w);
-  s->kbs_h = (int)ceil_div(kb_h, s->ws_h); s->ws_h = (int)ceil_div(kb_h, s->kbs_h);
   {
     const int64_t tiles = ceil_div(d.Lin, kD2Q * 1024) * d.B * s->ngroups;
     int64_t ws = std::max<int64_t>(1, std::min<int64_t>(d.C / 4 > 0 ? d.C / 4 : 1, ceil_div(148, tiles)));
     s->cps_h2 = (int)ceil_div(d.C, ws);
     s->ws_h2 = (int)ceil_div(d.C, s->cps_h2);
   }
-  const int hs = std::max(s->ws_h, s->ws_h2);
-  const int64_t pw = (int64_t)s->ws_w * d.C * d.R * d.T, ph = (int64_t)hs * d.B * d.R * d.Lin;
+  // staging layout of prep_w_kernel: shifts down to A8 + 1 - Tq
+  s->prep_F = (s->Tq - s->A8) / 8 + 2;
+  s->prep_S = s->Tq / 8 + s->prep_F;
+  s->smem = kernel_smem(d, s->Tq, s->prep_S);
+  const KernelSmem& k = s->smem;
+  if (std::max(std::max(k.recon2, k.dgrad2), std::max(k.wgrad, k.prep_w)) > 232448) {
+    delete s;
+    set_error("internal: tc_nmfd_create: the shared-memory stages exceed 227 KB for T = " + std::to_string(d.T));
+    return -1;
+  }
+  int rc = 0;
+  if (!rc) rc = raise_smem_limit(tcnmfd_recon2_kernel<false>, k.recon2);
+  if (!rc) rc = raise_smem_limit(tcnmfd_recon2_kernel<true>, k.recon2);
+  if (!rc) rc = raise_smem_limit(tcnmfd_dgrad2_kernel, k.dgrad2);
+  if (!rc) rc = raise_smem_limit(tcnmfd_wgrad_kernel, k.wgrad);
+  if (!rc) rc = raise_smem_limit(prep_w_kernel, k.prep_w);
+  if (rc) { delete s; return rc; }
+  const int64_t pw = (int64_t)s->ws_w * d.C * d.R * d.T, ph = (int64_t)s->ws_h2 * d.B * d.R * d.Lin;
   s->part_floats = pw > ph ? pw : ph;
-  s->loss_blocks = (int)std::max<int64_t>(ceil_div(d.L, kM) * ceil_div(d.C, kM) * d.B, ceil_div(d.L, 8 * kR2N) * ceil_div(d.C, 16) * d.B);
-  const size_t wbytes = (size_t)s->Cpad * d.R * s->Tp * 2, hbytes = (size_t)d.B * d.R * s->Lp * 2;
+  s->loss_blocks = (int)(ceil_div(d.L, 8 * kR2N) * ceil_div(d.C, 16) * d.B);
+  const size_t hbytes = (size_t)d.B * d.R * s->Lp * 2;
   const size_t pbytes = ((size_t)d.B * d.C + 1) * s->Lq * 2;
   cudaError_t e = cudaSuccess;
-  if (e == cudaSuccess) e = cudaMalloc(&s->Wr16, wbytes);
-  if (e == cudaSuccess) e = cudaMalloc(&s->Wf16, wbytes);
   const size_t wshbytes = (size_t)s->Cpad * 8 * d.R * s->Tq * 2;
   if (e == cudaSuccess) e = cudaMalloc(&s->Wsh16, wshbytes);
   if (e == cudaSuccess) e = cudaMemset(s->Wsh16, 0, wshbytes);
@@ -963,8 +870,6 @@ int tc_nmfd_create(TcNmfdState** out, const NmfdShape& d) {
   if (e == cudaSuccess) e = cudaMalloc(&s->kappa, sizeof(float));
   if (e == cudaSuccess) e = cudaMalloc(&s->vsum, 257 * sizeof(double));
   if (e == cudaSuccess) e = cudaMalloc(&s->loss_part, (size_t)s->loss_blocks * sizeof(double));
-  if (e == cudaSuccess) e = cudaMemset(s->Wr16, 0, wbytes);
-  if (e == cudaSuccess) e = cudaMemset(s->Wf16, 0, wbytes);
   if (e == cudaSuccess) e = cudaMemset(s->Hp16, 0, hbytes);
   if (e == cudaSuccess) e = cudaMemset(s->P16, 0, pbytes);
   if (e == cudaSuccess) e = cudaMemset(s->exps, 0, 4 * sizeof(int));
@@ -973,21 +878,9 @@ int tc_nmfd_create(TcNmfdState** out, const NmfdShape& d) {
     set_error(std::string("tc_nmfd_create: ") + cudaGetErrorString(e));
     return 2;
   }
-  {
-    const int nkk = s->Tq / kKB;
-    const uint32_t st_r = (((uint32_t)nkk * Smem::kTile + (uint32_t)(8 * kR2N + s->Tq) * 2) + 1023u) & ~1023u;
-    const uint32_t st_d = (((uint32_t)nkk * Smem::kTile + kD2Q * ((((uint32_t)(1024 + s->Tq) * 2) + 127u) & ~127u)) + 1023u) & ~1023u;
-    const bool fits = kD2Stages * std::max(st_r, st_d) + 2048 <= 232448u;
-    s->need_tile_copies = !fits || getenv("NMFB200_NMFD_RECON1") != nullptr || getenv("NMFB200_NMFD_DGRAD1") != nullptr;
-  }
-  int rc = 0;
-  rc |= make_tmap2(&s->tmWr, s->Wr16, s->Cpad, (int64_t)d.R * s->Tp, (int64_t)d.R * s->Tp, kM);
-  // dgrad reads Wf16 as (C R) rows of Tp columns, Rp16 rows per tile
-  const int Rp16 = (d.R + 15) & ~15;
-  rc |= make_tmap2(&s->tmWf, s->Wf16, (int64_t)s->Cpad * d.R, s->Tp, s->Tp, Rp16);
-  rc |= make_tmap2(&s->tmP, s->P16, (int64_t)d.B * d.C, s->Lq, s->Lq, kM);
-  rc |= make_tmap2(&s->tmWs, s->Ws16, (int64_t)s->Cpad * s->ngroups * 128, s->Tq, s->Tq, 128);
-  rc |= make_tmap2(&s->tmWsh, s->Wsh16, (int64_t)s->Cpad * 8, (int64_t)d.R * s->Tq, (int64_t)d.R * s->Tq, 128);
+  rc |= make_tmap(&s->tmP, s->P16, (int64_t)d.B * d.C, s->Lq, s->Lq, kM);
+  rc |= make_tmap(&s->tmWs, s->Ws16, (int64_t)s->Cpad * s->ngroups * 128, s->Tq, s->Tq, 128);
+  rc |= make_tmap(&s->tmWsh, s->Wsh16, (int64_t)s->Cpad * 8, (int64_t)d.R * s->Tq, (int64_t)d.R * s->Tq, 128);
   if (rc) { tc_nmfd_destroy(s); return 2; }
   *out = s;
   return 0;
@@ -1005,29 +898,6 @@ int tc_nmfd_set_target(TcNmfdState* s, const float* V, double* vsum_host, cudaSt
 }
 
 namespace {
-
-template <int KIND>
-int launch(TcNmfdState* s, const CUtensorMap& tm, dim3 grid, NmfdTcParams& p, cudaStream_t st) {
-  auto kern = tcnmfd_kernel<KIND>;
-  static bool attr = false;
-  const int smem = Smem::kTotal + 1024;
-  if (!attr) {
-    NMF_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    attr = true;
-  }
-  kern<<<grid, kThreads, smem, st>>>(tm, p);
-  NMF_LAUNCH_CHECK();
-  return 0;
-}
-
-NmfdTcParams base_params(TcNmfdState* s, const float* V) {
-  NmfdTcParams p{};
-  p.B = s->d.B; p.C = s->d.C; p.L = s->d.L; p.R = s->d.R; p.T = s->d.T; p.Lin = s->d.Lin; p.Tp = s->Tp;
-  p.Lp = s->Lp; p.padl = s->padl; p.Lq = s->Lq;
-  p.Hp16 = s->Hp16; p.P16 = s->P16; p.P16out = s->P16; p.V = V; p.exps = s->exps; p.kappa = s->kappa;
-  p.out = s->part; p.loss_part = s->loss_part; p.nsplit = 1; p.kb_per_split = 0;
-  return p;
-}
 
 // arguments of the fold launch after a preparation launch: fold `outer x R x inner` partial sums into colsum[which], then kappa if this is the
 // last refresh of the call
@@ -1049,21 +919,9 @@ int refresh(TcNmfdState* s, const float* W, const float* H, cudaStream_t st) {
       NMF_LAUNCH_CHECK();
       s->aw_valid = true;
     }
-    // the reversed / forward copies are only read by the Toeplitz-tile kernels (A/B switches, or shifts too long for the
-    // eight-phase kernels' shared-memory stages)
-    const bool tile_copies = s->need_tile_copies;
-    // staging layout of prep_w_kernel: S slots per shift-residue class, F of them leading zeros (shifts down to A8 + 1 - Tq)
-    const int F = (s->Tq - s->A8) / 8 + 2, S = s->Tq / 8 + F;
-    const size_t wrow_bytes = (size_t)d.R * 8 * S * sizeof(float);
-    const int use_smem = (wrow_bytes <= 200 * 1024 && (int64_t)d.R * d.T < 65536) ? 1 : 0;
-    static size_t attr_bytes = 0;
-    if (use_smem && wrow_bytes > 48 * 1024 && wrow_bytes > attr_bytes) {
-      NMF_CUDA_CHECK(cudaFuncSetAttribute(prep_w_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wrow_bytes));
-      attr_bytes = wrow_bytes;
-    }
-    prep_w_kernel<<<d.C, 256, use_smem ? wrow_bytes : 0, st>>>(W, d.C, d.R, d.T, s->Tp, s->Tq, s->ngroups, s->absmax, s->exps,
-                                                               tile_copies ? s->Wr16 : nullptr, s->Wf16, s->Ws16, s->Wsh16,
-                                                               s->A8, s->cs_part, use_smem, S, F);
+    prep_w_kernel<<<d.C, 256, s->smem.prep_w, st>>>(W, d.C, d.R, d.T, s->Tq, s->ngroups, s->absmax, s->exps, s->Ws16,
+                                                    s->Wsh16, s->A8, s->cs_part, s->smem.prep_w > 0 ? 1 : 0, s->prep_S,
+                                                    s->prep_F);
     NMF_LAUNCH_CHECK();
     fold_colsum_kernel<<<d.R, 256, 0, st>>>(fold_tail_args(s, 0, d.C, 1, /*do_kappa=*/s->h_fresh));
     NMF_LAUNCH_CHECK();
@@ -1093,83 +951,46 @@ int tc_nmfd_recon(TcNmfdState* s, const float* V, const float* W, const float* H
                   cudaStream_t st) {
   int rc = refresh(s, W, H, st);
   if (rc) return rc;
-  static const bool v1 = getenv("NMFB200_NMFD_RECON1") != nullptr;      // A/B: the Toeplitz-tile formulation
-  const int nkk = s->Tq / kKB;
-  const uint32_t stage2 = (((uint32_t)nkk * Smem::kTile + (uint32_t)(8 * kR2N + s->Tq) * 2) + 1023u) & ~1023u;
-  const int smem2 = (int)(kD2Stages * stage2 + 8 * (2 * kD2Stages + 1) + 16 + 64 + 1024);
-  if (!v1 && smem2 <= 232448) {
-    const NmfdShape& d = s->d;
-    Recon2Params q{};
-    q.B = d.B; q.C = d.C; q.L = d.L; q.R = d.R; q.Lp = s->Lp; q.padl = s->padl; q.Lq = s->Lq; q.Tq = s->Tq; q.A8 = s->A8;
-    q.nks = (int)ceil_div(s->A8 + 8, 16);
-    q.Hp16 = s->Hp16; q.P16out = s->P16; q.V = V; q.exps = s->exps; q.kappa = s->kappa; q.loss_part = s->loss_part;
-    static int attr0 = 0, attr1 = 0;
-    int& attr = loss ? attr1 : attr0;
-    if (smem2 > attr) {
-      if (loss) NMF_CUDA_CHECK(cudaFuncSetAttribute(tcnmfd_recon2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
-      else NMF_CUDA_CHECK(cudaFuncSetAttribute(tcnmfd_recon2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
-      attr = smem2;
-    }
-    dim3 grid2((unsigned)ceil_div(d.L, 8 * kR2N), (unsigned)ceil_div(d.C, 16), (unsigned)d.B);
-    if (loss) {
-      tcnmfd_recon2_kernel<true><<<grid2, kD2Threads, smem2, st>>>(s->tmWsh, q);
-      NMF_LAUNCH_CHECK();
-      return sum_partials(s->loss_part, (int)(grid2.x * grid2.y * grid2.z), loss_dev, st);
-    }
-    tcnmfd_recon2_kernel<false><<<grid2, kD2Threads, smem2, st>>>(s->tmWsh, q);
-    NMF_LAUNCH_CHECK();
-    return 0;
-  }
-  NmfdTcParams p = base_params(s, V);
-  dim3 grid((unsigned)ceil_div(s->d.L, kM), (unsigned)ceil_div(s->d.C, kM), (unsigned)s->d.B);
+  const NmfdShape& d = s->d;
+  Recon2Params q{};
+  q.B = d.B; q.C = d.C; q.L = d.L; q.R = d.R; q.Lp = s->Lp; q.padl = s->padl; q.Lq = s->Lq; q.Tq = s->Tq; q.A8 = s->A8;
+  q.nks = (int)ceil_div(s->A8 + 8, 16);
+  q.Hp16 = s->Hp16; q.P16out = s->P16; q.V = V; q.exps = s->exps; q.kappa = s->kappa; q.loss_part = s->loss_part;
+  dim3 grid((unsigned)ceil_div(d.L, 8 * kR2N), (unsigned)ceil_div(d.C, 16), (unsigned)d.B);
   if (loss) {
-    rc = launch<kReconLoss>(s, s->tmWr, grid, p, st);
-    if (rc) return rc;
+    tcnmfd_recon2_kernel<true><<<grid, kD2Threads, s->smem.recon2, st>>>(s->tmWsh, q);
+    NMF_LAUNCH_CHECK();
     return sum_partials(s->loss_part, (int)(grid.x * grid.y * grid.z), loss_dev, st);
   }
-  return launch<kRecon>(s, s->tmWr, grid, p, st);
+  tcnmfd_recon2_kernel<false><<<grid, kD2Threads, s->smem.recon2, st>>>(s->tmWsh, q);
+  NMF_LAUNCH_CHECK();
+  return 0;
 }
 
 // numerator partials of the W update from the P16 written by the last recon: [*nsplit][C][R][T] fp32
 int tc_nmfd_wgrad(TcNmfdState* s, const float** part, int* nsplit, cudaStream_t st) {
-  NmfdTcParams p = base_params(s, nullptr);
-  p.nsplit = s->ws_w; p.kb_per_split = s->kbs_w;
-  dim3 grid((unsigned)ceil_div(s->d.C, kM), (unsigned)s->d.R, (unsigned)s->ws_w);
-  int rc = launch<kWgrad>(s, s->tmP, grid, p, st);
+  const NmfdShape& d = s->d;
+  WgradParams p{};
+  p.B = d.B; p.C = d.C; p.L = d.L; p.R = d.R; p.T = d.T; p.Lp = s->Lp; p.padl = s->padl;
+  p.Hp16 = s->Hp16; p.exps = s->exps; p.out = s->part; p.kb_per_split = s->kbs_w;
+  dim3 grid((unsigned)ceil_div(d.C, kM), (unsigned)d.R, (unsigned)s->ws_w);
+  tcnmfd_wgrad_kernel<<<grid, kThreads, s->smem.wgrad, st>>>(s->tmP, p);
+  NMF_LAUNCH_CHECK();
   *part = s->part; *nsplit = s->ws_w;
-  return rc;
+  return 0;
 }
 
 int tc_nmfd_dgrad(TcNmfdState* s, const float** part, int* nsplit, cudaStream_t st) {
-  static const bool v1 = getenv("NMFB200_NMFD_DGRAD1") != nullptr;      // A/B: the Toeplitz-tile formulation
-  if (!v1) {
-    const NmfdShape& d = s->d;
-    Dgrad2Params q{};
-    q.B = d.B; q.C = d.C; q.R = d.R; q.Lin = d.Lin; q.Lq = s->Lq; q.Tq = s->Tq; q.ngroups = s->ngroups;
-    q.P16 = s->P16; q.exps = s->exps; q.out = s->part; q.c_per_split = s->cps_h2;
-    q.nks = (int)ceil_div(d.T + 7, 16);
-    const int nkk = s->Tq / kKB;
-    const uint32_t seg_pitch = (((uint32_t)(1024 + s->Tq) * 2) + 127u) & ~127u;
-    const uint32_t stage = (((uint32_t)nkk * Smem::kTile + kD2Q * seg_pitch) + 1023u) & ~1023u;
-    const int smem = (int)(kD2Stages * stage + 8 * (2 * kD2Stages + 1) + 16 + 1024);
-    if (smem > 232448) { set_error("nmfd dgrad: shift extent too large for the shared-memory stages"); return 1; }
-    static int attr_smem = 0;
-    if (smem > attr_smem) {
-      NMF_CUDA_CHECK(cudaFuncSetAttribute(tcnmfd_dgrad2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-      attr_smem = smem;
-    }
-    dim3 grid((unsigned)ceil_div(d.Lin, kD2Q * 1024), (unsigned)s->ws_h2, (unsigned)(d.B * s->ngroups));
-    tcnmfd_dgrad2_kernel<<<grid, kD2Threads, smem, st>>>(s->tmWs, q);
-    NMF_LAUNCH_CHECK();
-    *part = s->part; *nsplit = s->ws_h2;
-    return 0;
-  }
-  NmfdTcParams p = base_params(s, nullptr);
-  p.nsplit = s->ws_h; p.kb_per_split = s->kbs_h;
-  dim3 grid((unsigned)ceil_div(s->d.Lin, kM), (unsigned)s->ws_h, (unsigned)s->d.B);
-  int rc = launch<kDgrad>(s, s->tmWf, grid, p, st);
-  *part = s->part; *nsplit = s->ws_h;
-  return rc;
+  const NmfdShape& d = s->d;
+  Dgrad2Params q{};
+  q.B = d.B; q.C = d.C; q.R = d.R; q.Lin = d.Lin; q.Lq = s->Lq; q.Tq = s->Tq; q.ngroups = s->ngroups;
+  q.P16 = s->P16; q.exps = s->exps; q.out = s->part; q.c_per_split = s->cps_h2;
+  q.nks = (int)ceil_div(d.T + 7, 16);
+  dim3 grid((unsigned)ceil_div(d.Lin, kD2Q * 1024), (unsigned)s->ws_h2, (unsigned)(d.B * s->ngroups));
+  tcnmfd_dgrad2_kernel<<<grid, kD2Threads, s->smem.dgrad2, st>>>(s->tmWs, q);
+  NMF_LAUNCH_CHECK();
+  *part = s->part; *nsplit = s->ws_h2;
+  return 0;
 }
 
 const float* tc_nmfd_kappa(const TcNmfdState* s) { return s->kappa; }
@@ -1190,17 +1011,6 @@ void tc_nmfd_mark_dirty(TcNmfdState* s) {
   s->aw_valid = s->ah_valid = false;
 }
 
-// report (and clear) a recorded mbarrier wait abort of the NMFD kernels; the caller has synchronised the stream
-int tc_nmfd_check_wait_abort() {
-  unsigned int h[8] = {0};
-  if (cudaMemcpyFromSymbol(h, ptx::g_wait_abort, sizeof(h)) != cudaSuccess) return -1;
-  if (h[0]) {
-    fprintf(stderr, "nmf_b200: NMFD mbarrier wait aborted: block %u thread %u bar_addr %u parity %u\n", h[1], h[2], h[3], h[4]);
-    unsigned int z[8] = {0};
-    cudaMemcpyToSymbol(ptx::g_wait_abort, z, sizeof(z));
-    return 1;
-  }
-  return 0;
-}
+int tc_nmfd_check_wait_abort() { return ptx::check_wait_abort("NMFD "); }
 
 }  // namespace nmfb200

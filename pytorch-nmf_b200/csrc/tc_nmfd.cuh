@@ -1,4 +1,4 @@
-// NMFD on tcgen05 tensor cores (beta = 1): sliding GEMMs with a Toeplitz operand built in shared memory -- interface used by
+// NMFD on tcgen05 tensor cores (beta = 1): im2col-free sliding GEMMs for kernels of up to 128 shifts -- interface used by
 // capi.cu.  See tc_nmfd.cu.
 #pragma once
 #include "common.cuh"
@@ -7,7 +7,8 @@ namespace nmfb200 {
 
 struct TcNmfdState;
 
-bool tc_nmfd_supported(const NmfdShape& d, double beta);
+// shapes the kernels compute: one sliding axis, T <= 128 (every shift of wgrad in one accumulator), R <= 256
+bool tc_nmfd_shape_supported(const NmfdShape& d);
 int tc_nmfd_create(TcNmfdState** out, const NmfdShape& d);
 void tc_nmfd_destroy(TcNmfdState* s);
 // sum(V) for the centring constant kappa (also returned to the host: synchronises `st`)
