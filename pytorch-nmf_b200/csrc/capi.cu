@@ -109,17 +109,14 @@ void free_ctx(nmfb200_ctx* c) {
   delete c;
 }
 
-// CUDA-core contraction of one NMF factor update into c->num / c->den (chunked partials).
-int simt_contract_w(nmfb200_ctx* c, const float* W, const float* H, double beta, cudaStream_t st) {
-  // F = W (C rows), G = H (N rows), Vm = V^T
+// CUDA-core contraction of one NMF factor update (which = 0: W, 1: H) into c->num / c->den (chunked partials).
+int simt_contract(nmfb200_ctx* c, int which, const float* W, const float* H, double beta, cudaStream_t st) {
   if (beta != 1.0) { int e = ensure_den(c); if (e) return e; }
-  return simt_nmf_contract(c->V, c->ldv, /*trans=*/1, W, H, c->C, c->N, (int)c->R, beta, c->nch_w, c->num,
-                           c->den, c->R, c->C * c->R, st);
-}
-int simt_contract_h(nmfb200_ctx* c, const float* W, const float* H, double beta, cudaStream_t st) {
-  if (beta != 1.0) { int e = ensure_den(c); if (e) return e; }
-  return simt_nmf_contract(c->V, c->ldv, /*trans=*/0, H, W, c->N, c->C, (int)c->R, beta, c->nch_h, c->num,
-                           c->den, c->R, c->N * c->R, st);
+  // W update: F = W (C rows), G = H (N rows), Vm = V^T;  H update: F = H, G = W, Vm = V
+  const int64_t rows = which == 0 ? c->C : c->N;
+  return simt_nmf_contract(c->V, c->ldv, /*trans=*/which == 0 ? 1 : 0, which == 0 ? W : H, which == 0 ? H : W, rows,
+                           which == 0 ? c->N : c->C, (int)c->R, beta, which == 0 ? c->nch_w : c->nch_h, c->num, c->den,
+                           c->R, rows * c->R, st);
 }
 
 bool use_tc(const nmfb200_ctx* c, double beta) {
@@ -291,36 +288,88 @@ int nmfb200_nmf_set_target_sparse(nmfb200_ctx* ctx, int64_t nnz, const int64_t* 
 }
 
 namespace {
-// one factor update on the compressed form whose segments are that factor's rows (which = 0: W over CSC, 1: H over CSR)
-int sparse_update(nmfb200_ctx* ctx, int which, float* F, const float* other, double beta, double gamma, double l1_reg,
-                  double l2_reg, cudaStream_t st) {
-  if (beta != 1.0 && beta != 2.0) return fail(NMFB200_ERR_INVALID, "sparse targets: beta must be 1 or 2 (densify the target for other beta)");
+// The ratio stage's input for one dense-NMF factor (which = 0: W, 1: H; rows x R, row pitch R): `nchunks` slabs of partial
+// numerators (and denominators, beta != 1) or, for beta 1, the column sum `kl` of the other factor as the denominator.
+ApplyArgs nmf_apply_args(const nmfb200_ctx* ctx, int which, const float* num, const float* den, const float* kl,
+                         int nchunks) {
+  ApplyArgs a{};
+  a.numel = (which == 0 ? ctx->C : ctx->N) * ctx->R; a.R = (int)ctx->R; a.inner = 1; a.rowlen = ctx->R; a.ldp = ctx->R;
+  a.num = num; a.den = den; a.kl_den = kl; a.nchunks = nchunks; a.chunk_stride = a.numel;
+  return a;
+}
+
+// Both terms of one dense-NMF factor update (which = 0: W, 1: H) from the current factors, described as the ratio stage's
+// input.  Dense target: the CUDA-core contraction's chunked partials.  Sparse target: the numerator at the non-zeros of the
+// compressed form whose segments are that factor's rows (W over CSC, H over CSR), and for beta 2 the denominator as the
+// factor's rows times the Gram matrix of the other factor (nmf.py:609).  Beta 1 divides by the column sum of the other
+// factor (nmf.py:122-131).  Shared by the update and by nmfb200_nmf_raw_terms; the tensor-core path has its own fused
+// ratio stage.
+int nmf_terms(nmfb200_ctx* ctx, const float* W, const float* H, int which, double beta, ApplyArgs& a, cudaStream_t st) {
   const int R = (int)ctx->R;
   const int64_t rows = which == 0 ? ctx->C : ctx->N, orows = which == 0 ? ctx->N : ctx->C;
-  const int64_t* ptr = which == 0 ? ctx->sp_ccol : ctx->sp_crow;
-  const int64_t* idx = which == 0 ? ctx->sp_row : ctx->sp_col;
-  const float* val = which == 0 ? ctx->sp_val_t : ctx->sp_val;
-  int rc = sparse_numerator(ptr, idx, val, F, other, R, rows, beta, ctx->num, st);
+  const float* other = which == 0 ? H : W;
+  int rc, nchunks = 1;
+  if (ctx->sparse) {
+    if (beta != 1.0 && beta != 2.0) return fail(NMFB200_ERR_INVALID, "sparse targets: beta must be 1 or 2 (densify the target for other beta)");
+    const int64_t* ptr = which == 0 ? ctx->sp_ccol : ctx->sp_crow;
+    const int64_t* idx = which == 0 ? ctx->sp_row : ctx->sp_col;
+    const float* val = which == 0 ? ctx->sp_val_t : ctx->sp_val;
+    const float* F = which == 0 ? W : H;
+    rc = sparse_numerator(ptr, idx, val, F, other, R, rows, beta, ctx->num, st);
+    if (rc == 0 && beta == 2.0) {
+      rc = ensure_den(ctx);
+      if (rc) return rc;
+      float* G = ctx->sp_gram + (1 - which) * R * R;
+      rc = sparse_gram(other, orows, R, ctx->sp_gram + 2 * R * R, G, st);
+      if (rc == 0) rc = sparse_rows_times_gram(F, G, rows, R, ctx->den, st);
+    }
+  } else {
+    nchunks = which == 0 ? ctx->nch_w : ctx->nch_h;
+    rc = simt_contract(ctx, which, W, H, beta, st);
+  }
   if (rc) return rc;
   float* kl = nullptr;
   if (beta == 1.0) {
-    kl = ctx->colsum + (1 - which) * R;                        // colsum of the OTHER factor, nmf.py:122-131
+    kl = ctx->colsum + (1 - which) * R;
     rc = factor_colsum(other, orows, R, 1, ctx->cs_scratch, ctx->cs_scratch_floats, kl, st);
-  } else {
-    rc = ensure_den(ctx);
     if (rc) return rc;
-    float* G = ctx->sp_gram + (1 - which) * R * R;             // Gram matrix of the other factor
-    rc = sparse_gram(other, orows, R, ctx->sp_gram + 2 * R * R, G, st);
-    if (rc) return rc;
-    rc = sparse_rows_times_gram(F, G, rows, R, ctx->den, st);  // nmf.py:609
   }
+  a = nmf_apply_args(ctx, which, ctx->num, beta == 1.0 ? nullptr : ctx->den, kl, nchunks);
+  return 0;
+}
+
+// nmf.py:78-92 on the terms `a` of one factor; the tensor-core operand copy of that factor is stale afterwards.
+int nmf_apply(nmfb200_ctx* ctx, int which, ApplyArgs a, float* param, double gamma, double l1_reg, double l2_reg,
+              cudaStream_t st) {
+  a.param = param; a.gamma = (float)gamma; a.l1 = (float)l1_reg; a.l2 = (float)l2_reg;
+  int rc = apply_update(a, st);
   if (rc) return rc;
-  ApplyArgs a{};
-  a.param = F; a.numel = rows * R; a.R = R; a.inner = 1; a.rowlen = R;
-  a.num = ctx->num; a.den = beta == 1.0 ? nullptr : ctx->den; a.nchunks = 1; a.chunk_stride = 0;
-  a.ldp = R; a.kl_den = kl; a.out_scale = nullptr;
-  a.gamma = (float)gamma; a.l1 = (float)l1_reg; a.l2 = (float)l2_reg; a.absmax_bits = nullptr;
-  return apply_update(a, st);
+  if (ctx->tc) tc_mark_dirty(ctx->tc, which == 0, which == 1);
+  return 0;
+}
+
+int nmf_update(nmfb200_ctx* ctx, const float* W, const float* H, int which, float* param, double beta, double gamma,
+               double l1_reg, double l2_reg, cudaStream_t st) {
+  if (use_tc(ctx, beta))
+    return which == 0 ? tc_update_w(ctx->tc, param, H, beta, gamma, l1_reg, l2_reg, st)
+                      : tc_update_h(ctx->tc, W, param, beta, gamma, l1_reg, l2_reg, st);
+  ApplyArgs a;
+  int rc = nmf_terms(ctx, W, H, which, beta, a, st);
+  if (rc) return rc;
+  return nmf_apply(ctx, which, a, param, gamma, l1_reg, l2_reg, st);
+}
+
+// nmfb200_nmf_raw_terms past its argument checks: [numerator rows x R | colsum(other) R (beta 1) or denominator rows x R]
+int nmf_raw_terms(nmfb200_ctx* ctx, const float* W, const float* H, int which, double beta, float* out, cudaStream_t st) {
+  if (use_tc(ctx, beta) && tc_supports_partial(ctx->tc, beta)) return tc_raw_terms(ctx->tc, which, W, H, beta, out, st);
+  ApplyArgs a;
+  int rc = nmf_terms(ctx, W, H, which, beta, a, st);
+  if (rc) return rc;
+  rc = raw_sum(a, out, out + a.numel, st);
+  if (rc) return rc;
+  if (beta == 1.0)
+    NMF_CUDA_CHECK(cudaMemcpyAsync(out + a.numel, a.kl_den, (size_t)ctx->R * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  return 0;
 }
 
 int sparse_loss_ctx(nmfb200_ctx* ctx, const float* W, const float* H, double beta, double* loss_dev, cudaStream_t st) {
@@ -368,26 +417,7 @@ int nmfb200_nmf_update_w(nmfb200_ctx* ctx, float* W, const float* H, double beta
   CTX_GUARD(ctx, 0);
   if (!ctx->has_target) return fail(NMFB200_ERR_STATE, "set_target has not been called");
   if (!W || !H) return fail(NMFB200_ERR_INVALID, "null factor pointer");
-  cudaStream_t st = (cudaStream_t)stream;
-  if (ctx->sparse) return sparse_update(ctx, 0, W, H, beta, gamma, l1_reg, l2_reg, st);
-  if (use_tc(ctx, beta)) return tc_update_w(ctx->tc, W, H, beta, gamma, l1_reg, l2_reg, st);
-  int rc = simt_contract_w(ctx, W, H, beta, st);
-  if (rc) return rc;
-  float* kl = nullptr;
-  if (beta == 1.0) {
-    kl = ctx->colsum + ctx->R;
-    rc = factor_colsum(H, ctx->N, (int)ctx->R, 1, ctx->cs_scratch, ctx->cs_scratch_floats, kl, st);
-    if (rc) return rc;
-  }
-  ApplyArgs a{};
-  a.param = W; a.numel = ctx->C * ctx->R; a.R = (int)ctx->R; a.inner = 1; a.rowlen = ctx->R;
-  a.num = ctx->num; a.den = beta == 1.0 ? nullptr : ctx->den; a.nchunks = ctx->nch_w;
-  a.chunk_stride = ctx->C * ctx->R; a.ldp = ctx->R; a.kl_den = kl; a.out_scale = nullptr;
-  a.gamma = (float)gamma; a.l1 = (float)l1_reg; a.l2 = (float)l2_reg; a.absmax_bits = nullptr;
-  rc = apply_update(a, st);
-  if (rc) return rc;
-  if (ctx->tc) tc_mark_dirty(ctx->tc, true, false);
-  return 0;
+  return nmf_update(ctx, W, H, 0, W, beta, gamma, l1_reg, l2_reg, (cudaStream_t)stream);
 }
 
 int nmfb200_nmf_update_h(nmfb200_ctx* ctx, const float* W, float* H, double beta, double gamma, double l1_reg,
@@ -395,26 +425,7 @@ int nmfb200_nmf_update_h(nmfb200_ctx* ctx, const float* W, float* H, double beta
   CTX_GUARD(ctx, 0);
   if (!ctx->has_target) return fail(NMFB200_ERR_STATE, "set_target has not been called");
   if (!W || !H) return fail(NMFB200_ERR_INVALID, "null factor pointer");
-  cudaStream_t st = (cudaStream_t)stream;
-  if (ctx->sparse) return sparse_update(ctx, 1, H, W, beta, gamma, l1_reg, l2_reg, st);
-  if (use_tc(ctx, beta)) return tc_update_h(ctx->tc, W, H, beta, gamma, l1_reg, l2_reg, st);
-  int rc = simt_contract_h(ctx, W, H, beta, st);
-  if (rc) return rc;
-  float* kl = nullptr;
-  if (beta == 1.0) {
-    kl = ctx->colsum;
-    rc = factor_colsum(W, ctx->C, (int)ctx->R, 1, ctx->cs_scratch, ctx->cs_scratch_floats, kl, st);
-    if (rc) return rc;
-  }
-  ApplyArgs a{};
-  a.param = H; a.numel = ctx->N * ctx->R; a.R = (int)ctx->R; a.inner = 1; a.rowlen = ctx->R;
-  a.num = ctx->num; a.den = beta == 1.0 ? nullptr : ctx->den; a.nchunks = ctx->nch_h;
-  a.chunk_stride = ctx->N * ctx->R; a.ldp = ctx->R; a.kl_den = kl; a.out_scale = nullptr;
-  a.gamma = (float)gamma; a.l1 = (float)l1_reg; a.l2 = (float)l2_reg; a.absmax_bits = nullptr;
-  rc = apply_update(a, st);
-  if (rc) return rc;
-  if (ctx->tc) tc_mark_dirty(ctx->tc, false, true);
-  return 0;
+  return nmf_update(ctx, W, H, 1, H, beta, gamma, l1_reg, l2_reg, (cudaStream_t)stream);
 }
 
 int nmfb200_nmf_iterate(nmfb200_ctx* ctx, float* W, float* H, double beta, double gamma, double l1_reg,
@@ -422,11 +433,11 @@ int nmfb200_nmf_iterate(nmfb200_ctx* ctx, float* W, float* H, double beta, doubl
   CTX_GUARD(ctx, 0);
   if (!ctx->has_target) return fail(NMFB200_ERR_STATE, "set_target has not been called");
   if (!W || !H || n_iter < 0) return fail(NMFB200_ERR_INVALID, "bad argument");
-  if (use_tc(ctx, beta)) return tc_iterate(ctx->tc, W, H, beta, gamma, l1_reg, l2_reg, n_iter, (cudaStream_t)stream);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (use_tc(ctx, beta)) return tc_iterate(ctx->tc, W, H, beta, gamma, l1_reg, l2_reg, n_iter, st);
   for (int i = 0; i < n_iter; ++i) {
-    int rc = nmfb200_nmf_update_w(ctx, W, H, beta, gamma, l1_reg, l2_reg, stream);
-    if (rc) return rc;
-    rc = nmfb200_nmf_update_h(ctx, W, H, beta, gamma, l1_reg, l2_reg, stream);
+    int rc = nmf_update(ctx, W, H, 0, W, beta, gamma, l1_reg, l2_reg, st);
+    if (rc == 0) rc = nmf_update(ctx, W, H, 1, H, beta, gamma, l1_reg, l2_reg, st);
     if (rc) return rc;
   }
   return 0;
@@ -439,7 +450,7 @@ int nmfb200_nmf_loss(nmfb200_ctx* ctx, const float* W, const float* H, double be
   if (!W || !H || !loss_dev) return fail(NMFB200_ERR_INVALID, "null pointer");
   cudaStream_t st = (cudaStream_t)stream;
   if (ctx->sparse) return sparse_loss_ctx(ctx, W, H, beta, loss_dev, st);
-  if (use_tc(ctx, beta) && tc_supports_loss(ctx->tc, beta)) return tc_loss(ctx->tc, W, H, beta, loss_dev, st);
+  if (use_tc(ctx, beta)) return tc_loss(ctx->tc, W, H, beta, loss_dev, st);
   return simt_nmf_loss(ctx->V, ctx->ldv, H, W, ctx->N, ctx->C, (int)ctx->R, beta, ctx->loss_blocks,
                        ctx->loss_max_blocks, loss_dev, st);
 }
@@ -449,32 +460,9 @@ int nmfb200_nmf_loss_prefetch_w(nmfb200_ctx* ctx, const float* W, const float* H
   CTX_GUARD(ctx, 0);
   if (!ctx->has_target) return fail(NMFB200_ERR_STATE, "set_target has not been called");
   if (!W || !H || !loss_dev) return fail(NMFB200_ERR_INVALID, "null pointer");
-  if (!ctx->sparse && use_tc(ctx, beta) && tc_supports_loss(ctx->tc, beta))
+  if (!ctx->sparse && use_tc(ctx, beta))
     return tc_loss_prefetch_w(ctx->tc, W, H, beta, loss_dev, (cudaStream_t)stream);
   return nmfb200_nmf_loss(ctx, W, H, beta, loss_dev, stream);
-}
-
-int64_t nmfb200_nmf_w_partial_numel(const nmfb200_ctx* ctx, double beta) {
-  if (!ctx || ctx->kind != 0) return -1;
-  return beta == 1.0 ? ctx->C * ctx->R + ctx->R : 2 * ctx->C * ctx->R;
-}
-
-int nmfb200_nmf_w_partial(nmfb200_ctx* ctx, const float* W, const float* H, double beta, float* partial,
-                          void* stream) {
-  CTX_GUARD(ctx, 0);
-  if (!ctx->has_target) return fail(NMFB200_ERR_STATE, "set_target has not been called");
-  if (ctx->sparse) return fail(NMFB200_ERR_STATE, "not available for a sparse target");
-  if (!W || !H || !partial) return fail(NMFB200_ERR_INVALID, "null pointer");
-  cudaStream_t st = (cudaStream_t)stream;
-  if (use_tc(ctx, beta) && tc_supports_partial(ctx->tc, beta)) return tc_w_partial(ctx->tc, W, H, beta, partial, st);
-  int rc = simt_contract_w(ctx, W, H, beta, st);
-  if (rc) return rc;
-  const int64_t CR = ctx->C * ctx->R;
-  rc = reduce_chunks(ctx->num, ctx->nch_w, CR, ctx->C, (int)ctx->R, ctx->R, partial, st);
-  if (rc) return rc;
-  if (beta == 1.0)
-    return factor_colsum(H, ctx->N, (int)ctx->R, 1, ctx->cs_scratch, ctx->cs_scratch_floats, partial + CR, st);
-  return reduce_chunks(ctx->den, ctx->nch_w, CR, ctx->C, (int)ctx->R, ctx->R, partial + CR, st);
 }
 
 int64_t nmfb200_nmf_raw_terms_numel(const nmfb200_ctx* ctx, int which, double beta) {
@@ -489,21 +477,19 @@ int nmfb200_nmf_raw_terms(nmfb200_ctx* ctx, const float* W, const float* H, int 
   if (!ctx->has_target) return fail(NMFB200_ERR_STATE, "set_target has not been called");
   if (ctx->sparse) return fail(NMFB200_ERR_STATE, "not available for a sparse target");
   if (!W || !H || !out || (which != 0 && which != 1)) return fail(NMFB200_ERR_INVALID, "bad argument");
-  cudaStream_t st = (cudaStream_t)stream;
-  if (use_tc(ctx, beta) && tc_supports_partial(ctx->tc, beta)) return tc_raw_terms(ctx->tc, which, W, H, beta, out, st);
-  int rc = which == 0 ? simt_contract_w(ctx, W, H, beta, st) : simt_contract_h(ctx, W, H, beta, st);
-  if (rc) return rc;
-  const int64_t rows = which == 0 ? ctx->C : ctx->N;
-  const int64_t RR = rows * ctx->R;
-  const int nch = which == 0 ? ctx->nch_w : ctx->nch_h;
-  rc = reduce_chunks(ctx->num, nch, RR, rows, (int)ctx->R, ctx->R, out, st);
-  if (rc) return rc;
-  if (beta == 1.0) {      // nmf.py:122-131: the KL denominator is the column sum of the OTHER factor
-    const float* other = which == 0 ? H : W;
-    return factor_colsum(other, which == 0 ? ctx->N : ctx->C, (int)ctx->R, 1, ctx->cs_scratch, ctx->cs_scratch_floats,
-                         out + RR, st);
-  }
-  return reduce_chunks(ctx->den, nch, RR, rows, (int)ctx->R, ctx->R, out + RR, st);
+  return nmf_raw_terms(ctx, W, H, which, beta, out, (cudaStream_t)stream);
+}
+
+// The sharded W update's partial is the W update's raw terms.
+int64_t nmfb200_nmf_w_partial_numel(const nmfb200_ctx* ctx, double beta) { return nmfb200_nmf_raw_terms_numel(ctx, 0, beta); }
+
+int nmfb200_nmf_w_partial(nmfb200_ctx* ctx, const float* W, const float* H, double beta, float* partial,
+                          void* stream) {
+  CTX_GUARD(ctx, 0);
+  if (!ctx->has_target) return fail(NMFB200_ERR_STATE, "set_target has not been called");
+  if (ctx->sparse) return fail(NMFB200_ERR_STATE, "not available for a sparse target");
+  if (!W || !H || !partial) return fail(NMFB200_ERR_INVALID, "null pointer");
+  return nmf_raw_terms(ctx, W, H, 0, beta, partial, (cudaStream_t)stream);
 }
 
 /* ---- row-sharded W update over peer memory (NVLink, one process per GPU) ---------------------- */
@@ -552,16 +538,9 @@ int nmfb200_nmf_w_apply(nmfb200_ctx* ctx, float* W, const float* reduced, double
   if (!W || !reduced) return fail(NMFB200_ERR_INVALID, "null pointer");
   cudaStream_t st = (cudaStream_t)stream;
   if (use_tc(ctx, beta)) return tc_w_apply(ctx->tc, W, reduced, beta, gamma, l1_reg, l2_reg, st);
-  const int64_t CR = ctx->C * ctx->R;
-  ApplyArgs a{};
-  a.param = W; a.numel = CR; a.R = (int)ctx->R; a.inner = 1; a.rowlen = ctx->R;
-  a.num = reduced; a.den = beta == 1.0 ? nullptr : reduced + CR; a.nchunks = 1; a.chunk_stride = 0;
-  a.ldp = ctx->R; a.kl_den = beta == 1.0 ? reduced + CR : nullptr; a.out_scale = nullptr;
-  a.gamma = (float)gamma; a.l1 = (float)l1_reg; a.l2 = (float)l2_reg; a.absmax_bits = nullptr;
-  int rc = apply_update(a, st);
-  if (rc) return rc;
-  if (ctx->tc) tc_mark_dirty(ctx->tc, true, false);
-  return 0;
+  const float* den = reduced + ctx->C * ctx->R;          // [numerator C x R | colsum(H) R (beta 1) or denominator C x R]
+  const ApplyArgs a = nmf_apply_args(ctx, 0, reduced, beta == 1.0 ? nullptr : den, beta == 1.0 ? den : nullptr, 1);
+  return nmf_apply(ctx, 0, a, W, gamma, l1_reg, l2_reg, st);
 }
 
 int nmfb200_nmf_contract_only(nmfb200_ctx* ctx, const float* W, const float* H, int which, double beta,
@@ -572,7 +551,7 @@ int nmfb200_nmf_contract_only(nmfb200_ctx* ctx, const float* W, const float* H, 
   if (!W || !H) return fail(NMFB200_ERR_INVALID, "null factor pointer");
   cudaStream_t st = (cudaStream_t)stream;
   if (use_tc(ctx, beta)) return tc_contract_only(ctx->tc, W, H, which, beta, st);
-  return which == 0 ? simt_contract_w(ctx, W, H, beta, st) : simt_contract_h(ctx, W, H, beta, st);
+  return simt_contract(ctx, which, W, H, beta, st);
 }
 
 /* ---- NMFD ------------------------------------------------------------------------------------ */
@@ -699,7 +678,7 @@ static int nmfd_terms(nmfb200_ctx* ctx, const float* W, const float* H, int whic
   const int64_t inner = which == 0 ? d.w_inner() : d.h_inner();
   a = ApplyArgs{};
   a.numel = (int64_t)(which == 0 ? d.C : d.B) * d.R * inner; a.R = d.R; a.inner = inner; a.rowlen = (int64_t)d.R * inner;
-  a.chunk_stride = a.numel; a.ldp = a.rowlen; a.out_scale = nullptr; a.absmax_bits = nullptr;
+  a.chunk_stride = a.numel; a.ldp = a.rowlen; a.absmax_bits = nullptr;
   *tc = nmfd_use_tc(ctx, beta);
   if (*tc) {
     int rc = tc_nmfd_recon(ctx->tcd, ctx->V, W, H, false, nullptr, st);

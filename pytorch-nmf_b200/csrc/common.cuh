@@ -84,7 +84,6 @@ struct ApplyArgs {
   float* param; int64_t numel; int R; int64_t inner; int64_t rowlen;
   const float* num; const float* den; int nchunks; int64_t chunk_stride; int64_t ldp;
   const float* kl_den;     // [R] when beta == 1 (den == nullptr)
-  const float* out_scale;  // device scalar multiplying num/den partials (nullptr = 1)
   float gamma, l1, l2;
   unsigned int* absmax_bits;  // optional: atomicMax of the updated values (non-negative floats)
   const float* kappa;         // optional (with kappa_vec): the partials hold sum (P - kappa) G; num += *kappa * kappa_vec[r]
@@ -97,9 +96,6 @@ int raw_sum(const ApplyArgs& a, float* num_out, float* den_out, cudaStream_t st)
 int factor_colsum(const float* x, int64_t outer, int R, int64_t inner, float* scratch, int64_t scratch_floats,
                   float* sums, cudaStream_t st);
 int64_t colsum_scratch_floats(int64_t outer, int R, int64_t inner);
-// dst[i] = sum_ch src[ch*stride + i]   (chunk reduction for the sharded partial buffers)
-int reduce_chunks(const float* src, int nchunks, int64_t chunk_stride, int64_t rows, int R, int64_t ldp,
-                  float* dst, cudaStream_t st);
 // min / max of a strided fp32 matrix (fit()'s validation), results in mm[0..1]
 int matrix_minmax(const float* V, int64_t rows, int64_t cols, int64_t ld, float* scratch2048, float* mm,
                   cudaStream_t st);

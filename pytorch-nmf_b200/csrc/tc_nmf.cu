@@ -1742,7 +1742,6 @@ bool tc_supports_beta(const TcState* s, double beta) {
   // other beta: two-output kernel (rank <= 64)
   return s->Rp == 64 && s->TN == 128;
 }
-bool tc_supports_loss(const TcState* s, double beta) { return tc_supports_beta(s, beta); }
 bool tc_supports_partial(const TcState* s, double beta) { return beta != 2.0 && tc_supports_beta(s, beta); }
 
 int tc_set_target(TcState* s, const float* V, int64_t ldv, const float* minmax_dev, cudaStream_t st) {
@@ -1883,18 +1882,16 @@ int apply_and_finish(TcState* s, int which, float* param, bool apply, const Plan
 
 int ensure_synced(TcState* s, const float* W, const float* H, double beta, cudaStream_t st) {
   if (!s->has_target) { set_error("tensor-core path: set_target has not been called"); return 3; }
-  const bool both = s->dirty_w && s->dirty_h;
   if (s->dirty_w) {
     int rc = apply_and_finish(s, 0, const_cast<float*>(W), false, nullptr, beta, 1, 0, 0, st);
     if (rc) return rc;
     s->dirty_w = false;
   }
-  if (s->dirty_h) {
+  if (s->dirty_h) {      // after a W refresh, this one recomputes exps[3] with both column sums valid
     int rc = apply_and_finish(s, 1, const_cast<float*>(H), false, nullptr, beta, 1, 0, 0, st);
     if (rc) return rc;
     s->dirty_h = false;
   }
-  (void)both;   // the second refresh recomputes exps[3] with both column sums valid
   return 0;
 }
 
@@ -2039,10 +2036,6 @@ int tc_raw_terms(TcState* s, int which, const float* W, const float* H, double b
       s->colsum + (1 - which) * s->R, s->kappa, out);
   NMF_LAUNCH_CHECK();
   return 0;
-}
-
-int tc_w_partial(TcState* s, const float* W, const float* H, double beta, float* partial, cudaStream_t st) {
-  return tc_raw_terms(s, 0, W, H, beta, partial, st);
 }
 
 // Sharded W update, second half: nmf.py:78-92 on the all-reduced buffer with the tensor-core path's own ratio-stage

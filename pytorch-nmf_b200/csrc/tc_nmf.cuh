@@ -11,7 +11,6 @@ bool tc_shape_supported(int64_t N, int64_t C, int64_t R);
 int tc_create(TcState** out, int device, int64_t N, int64_t C, int64_t R, bool split);
 void tc_destroy(TcState* s);
 bool tc_supports_beta(const TcState* s, double beta);
-bool tc_supports_loss(const TcState* s, double beta);
 // row-sharded partials: beta 2 keeps the fp32 contraction (its numerator needs the Gram matrix of the global H)
 bool tc_supports_partial(const TcState* s, double beta);
 // minmax_dev: device float[2] = {min(V), max(V)} already queued on `st`
@@ -28,8 +27,8 @@ int tc_update_h(TcState* s, const float* W, float* H, double beta, double gamma,
                 cudaStream_t st);
 int tc_iterate(TcState* s, float* W, float* H, double beta, double gamma, double l1, double l2, int n_iter,
                cudaStream_t st);
-int tc_w_partial(TcState* s, const float* W, const float* H, double beta, float* partial, cudaStream_t st);
-// the same for either factor (which = 0: W, 1: H): [numerator rows x R | colsum(other) R (beta 1) or denominator rows x R]
+// raw update terms of one factor (which = 0: W, 1: H; which = 0 is the row-sharded W update's partial):
+// [numerator rows x R | colsum(other) R (beta 1) or denominator rows x R]
 int tc_raw_terms(TcState* s, int which, const float* W, const float* H, double beta, float* out, cudaStream_t st);
 int tc_w_apply(TcState* s, float* W, const float* reduced, double beta, double gamma, double l1, double l2,
                cudaStream_t st);

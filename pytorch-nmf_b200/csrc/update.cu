@@ -14,17 +14,14 @@ apply_update_kernel(ApplyArgs a) {
     const int64_t col = idx - row * a.rowlen;
     const int64_t off = row * a.ldp + col;
     const int r = (int)((idx / a.inner) % a.R);
-    const float sc = a.out_scale ? *a.out_scale : 1.0f;
     float num = 0.f;
     for (int ch = 0; ch < a.nchunks; ++ch) num += a.num[ch * a.chunk_stride + off];
-    num *= sc;
     if (a.kappa) num = fmaf(*a.kappa, a.kappa_vec[r], num);
     const float p = a.param[idx];
     float pos;
     if (a.den) {
       float den = 0.f;
       for (int ch = 0; ch < a.nchunks; ++ch) den += a.den[ch * a.chunk_stride + off];
-      den *= sc;
       pos = fmaxf(den, 0.f) + kEps;                          // nmf.py:83
     } else {
       pos = a.kl_den[r];                                     // nmf.py:368-369 / :381-382 (no relu, no eps)
@@ -52,16 +49,14 @@ raw_sum_kernel(ApplyArgs a, float* __restrict__ num_out, float* __restrict__ den
   if (idx >= a.numel) return;
   const int64_t row = idx / a.rowlen;
   const int64_t off = row * a.ldp + (idx - row * a.rowlen);
-  const float sc = a.out_scale ? *a.out_scale : 1.0f;
   float num = 0.f;
   for (int ch = 0; ch < a.nchunks; ++ch) num += a.num[ch * a.chunk_stride + off];
-  num *= sc;
   if (a.kappa) num = fmaf(*a.kappa, a.kappa_vec[(int)((idx / a.inner) % a.R)], num);
   num_out[idx] = num;
   if (den_out) {
     float den = 0.f;
     for (int ch = 0; ch < a.nchunks; ++ch) den += a.den[ch * a.chunk_stride + off];
-    den_out[idx] = den * sc;
+    den_out[idx] = den;
   }
 }
 
@@ -112,18 +107,6 @@ __global__ void colsum_final_kernel(const float* __restrict__ partial, int64_t n
   sums[r] = t;
 }
 
-__global__ void __launch_bounds__(256)
-reduce_chunks_kernel(const float* __restrict__ src, int nchunks, int64_t chunk_stride, int64_t rows, int R,
-                     int64_t ldp, float* __restrict__ dst) {
-  const int64_t idx = (int64_t)blockIdx.x * 256 + threadIdx.x;
-  if (idx >= rows * R) return;
-  const int64_t row = idx / R;
-  const int r = (int)(idx - row * R);
-  float t = 0.f;
-  for (int ch = 0; ch < nchunks; ++ch) t += src[ch * chunk_stride + row * ldp + r];
-  dst[idx] = t;
-}
-
 __device__ __forceinline__ float nan_min(float a, float b) { return (a != a || b != b) ? NAN : fminf(a, b); }
 __device__ __forceinline__ float nan_max(float a, float b) { return (a != a || b != b) ? NAN : fmaxf(a, b); }
 
@@ -172,7 +155,6 @@ apply_update_vec4_kernel(ApplyArgs a) {
     const int64_t row = idx / a.rowlen;
     const int64_t off = row * a.ldp + (idx - row * a.rowlen);
     const int r = (int)((idx / a.inner) % a.R);
-    const float sc = a.out_scale ? *a.out_scale : 1.0f;
     float4 num = make_float4(0.f, 0.f, 0.f, 0.f);
     for (int ch = 0; ch < a.nchunks; ++ch) {
       const float4 t = *reinterpret_cast<const float4*>(a.num + ch * a.chunk_stride + off);
@@ -188,9 +170,8 @@ apply_update_vec4_kernel(ApplyArgs a) {
     const float klden = a.den ? 0.f : a.kl_den[r];
     float4 p = *reinterpret_cast<const float4*>(a.param + idx);
     auto one = [&](float pv, float n, float d) {
-      n *= sc;
       if (a.kappa) n = fmaf(*a.kappa, a.kappa_vec[r], n);
-      const float pos = a.den ? fmaxf(d * sc, 0.f) + kEps : klden;   // nmf.py:83 / :368-369
+      const float pos = a.den ? fmaxf(d, 0.f) + kEps : klden;   // nmf.py:83 / :368-369
       return mu_step(pv, n, pos, a.l1, a.l2, a.gamma);
     };
     p.x = one(p.x, num.x, den.x); p.y = one(p.y, num.y, den.y); p.z = one(p.z, num.z, den.z); p.w = one(p.w, num.w, den.w);
@@ -252,14 +233,6 @@ int factor_colsum(const float* x, int64_t outer, int R, int64_t inner, float* sc
   }
   NMF_LAUNCH_CHECK();
   colsum_final_kernel<<<(unsigned)ceil_div(R, 64), 64, 0, st>>>(scratch, nb, R, sums);
-  NMF_LAUNCH_CHECK();
-  return 0;
-}
-
-int reduce_chunks(const float* src, int nchunks, int64_t chunk_stride, int64_t rows, int R, int64_t ldp,
-                  float* dst, cudaStream_t st) {
-  reduce_chunks_kernel<<<(unsigned)ceil_div(rows * R, 256), 256, 0, st>>>(src, nchunks, chunk_stride, rows, R,
-                                                                         ldp, dst);
   NMF_LAUNCH_CHECK();
   return 0;
 }

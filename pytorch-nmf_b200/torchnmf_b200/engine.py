@@ -102,7 +102,7 @@ def release_workspaces():
 
 
 class _CudaEngine:
-    kind = None
+    kind = None          # "nmf" or "nmfd": the family of nmfb200_<kind>_* entry points the engine calls
 
     def __init__(self):
         self._lib = _capi.load()
@@ -138,6 +138,35 @@ class _CudaEngine:
             self.close()
         except Exception:
             pass
+
+    @property
+    def _dev_index(self):
+        return self.device.index if self.device.index is not None else torch.cuda.current_device()
+
+    def _call(self, name, *args):
+        """nmfb200_<kind>_<name>(ctx, *args, stream) on the engine's current stream; raises on an error code."""
+        _capi.check(getattr(self._lib, f"nmfb200_{self.kind}_{name}")(self._ctx, *args, _stream(self.device)))
+
+    def update_w(self, beta, gamma, l1_reg, l2_reg):
+        self._call("update_w", _ptr(self.W), _ptr(self.H), beta, gamma, l1_reg, l2_reg)
+
+    def update_h(self, beta, gamma, l1_reg, l2_reg):
+        self._call("update_h", _ptr(self.W), _ptr(self.H), beta, gamma, l1_reg, l2_reg)
+
+    def loss_tensor(self, beta):
+        self._call("loss", _ptr(self.W), _ptr(self.H), beta, _ptr(self._loss))
+        return self._loss
+
+    def raw_terms(self, which, beta):
+        """(numerator, denominator) of the update of W (which=0) or H (which=1) from the CURRENT factors, untouched, in
+        the factor's own shape; the denominator is (R,) for beta == 1 (the column sums of the other factor).  What
+        BetaMu.step, PLCA.fit and sparse_fit are built from (include/nmf_b200.h: nmfb200_nmf_raw_terms, _nmfd_raw_terms)."""
+        f = self.W if which == 0 else self.H
+        n = int(getattr(self._lib, f"nmfb200_{self.kind}_raw_terms_numel")(self._ctx, int(which), float(beta)))
+        buf = torch.empty(n, dtype=torch.float32, device=self.device)
+        self._call("raw_terms", _ptr(self.W), _ptr(self.H), int(which), float(beta), _ptr(buf))
+        num, den = buf[:f.numel()].view(f.shape), buf[f.numel():]
+        return num, (den if beta == 1 else den.view(f.shape))
 
     @property
     def precision(self):
@@ -179,9 +208,17 @@ class _CudaEngine:
             self.W, self.H = keep
 
 
-class CudaNmfEngine(_CudaEngine):
-    """Dense NMF on one GPU: V (N,C), W (C,R), H (N,R), all fp32 CUDA tensors (W, H updated in place)."""
+class _NmfEngine(_CudaEngine):
+    """What the dense and the sparse-target NMF engines share beyond _CudaEngine."""
     kind = "nmf"
+
+    def iterate(self, n_iter, beta, gamma, l1_reg, l2_reg):
+        """n_iter x (update_w; update_h) in one host call."""
+        self._call("iterate", _ptr(self.W), _ptr(self.H), beta, gamma, l1_reg, l2_reg, int(n_iter))
+
+
+class CudaNmfEngine(_NmfEngine):
+    """Dense NMF on one GPU: V (N,C), W (C,R), H (N,R), all fp32 CUDA tensors (W, H updated in place)."""
 
     def __init__(self, V, W, H, precision="auto"):
         super().__init__()
@@ -193,7 +230,7 @@ class CudaNmfEngine(_CudaEngine):
         assert W.shape == (C, R) and H.shape == (N, R)
         self.V, self.W, self.H = V, W, H
         self.N, self.C, self.R = N, C, R
-        dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
+        dev_index = self._dev_index
         self._acquire(("nmf", dev_index, N, C, R, precision),
                       lambda ref: self._lib.nmfb200_nmf_create(ref, dev_index, N, C, R, _capi.PRECISIONS[precision]))
         self._loss = torch.zeros(1, dtype=torch.float64, device=self.device)
@@ -202,24 +239,6 @@ class CudaNmfEngine(_CudaEngine):
 
     def sync(self):
         _capi.check(self._lib.nmfb200_nmf_sync_factors(self._ctx, _ptr(self.W), _ptr(self.H), _stream(self.device)))
-
-    def update_w(self, beta, gamma, l1_reg, l2_reg):
-        _capi.check(self._lib.nmfb200_nmf_update_w(self._ctx, _ptr(self.W), _ptr(self.H), beta, gamma, l1_reg,
-                                                   l2_reg, _stream(self.device)))
-
-    def update_h(self, beta, gamma, l1_reg, l2_reg):
-        _capi.check(self._lib.nmfb200_nmf_update_h(self._ctx, _ptr(self.W), _ptr(self.H), beta, gamma, l1_reg,
-                                                   l2_reg, _stream(self.device)))
-
-    def iterate(self, n_iter, beta, gamma, l1_reg, l2_reg):
-        """n_iter x (update_w; update_h) in one host call."""
-        _capi.check(self._lib.nmfb200_nmf_iterate(self._ctx, _ptr(self.W), _ptr(self.H), beta, gamma, l1_reg, l2_reg,
-                                                  int(n_iter), _stream(self.device)))
-
-    def loss_tensor(self, beta):
-        _capi.check(self._lib.nmfb200_nmf_loss(self._ctx, _ptr(self.W), _ptr(self.H), beta, _ptr(self._loss),
-                                               _stream(self.device)))
-        return self._loss
 
     def loss_prefetch_w(self, beta):
         """The loss at the current factors, taken out of the NEXT W update's contraction pass where the library can fold it
@@ -244,19 +263,6 @@ class CudaNmfEngine(_CudaEngine):
         _capi.check(self._lib.nmfb200_nmf_w_partial(self._ctx, _ptr(self.W), _ptr(self.H), beta, _ptr(buf),
                                                     _stream(self.device)))
         return buf
-
-    def raw_terms(self, which, beta):
-        """(numerator, denominator) of the update of W (which=0) or H (which=1) from the CURRENT factors, untouched:
-        numerator (rows, R); denominator (R,) for beta == 1 (the column sums of the other factor) else (rows, R).
-        What BetaMu.step and PLCA.fit are built from (include/nmf_b200.h: nmfb200_nmf_raw_terms)."""
-        n = int(self._lib.nmfb200_nmf_raw_terms_numel(self._ctx, int(which), float(beta)))
-        buf = torch.empty(n, dtype=torch.float32, device=self.device)
-        _capi.check(self._lib.nmfb200_nmf_raw_terms(self._ctx, _ptr(self.W), _ptr(self.H), int(which), float(beta),
-                                                    _ptr(buf), _stream(self.device)))
-        rows = self.C if which == 0 else self.N
-        num = buf[:rows * self.R].view(rows, self.R)
-        den = buf[rows * self.R:]
-        return num, (den if beta == 1 else den.view(rows, self.R))
 
     # ---- row-sharded W update over peer memory (include/nmf_b200.h: nmfb200_nmf_peer_*) ----
     def peer_supported(self, beta):
@@ -286,11 +292,10 @@ class CudaNmfEngine(_CudaEngine):
                                                   l2_reg, _stream(self.device)))
 
 
-class CudaSparseNmfEngine(_CudaEngine):
+class CudaSparseNmfEngine(_NmfEngine):
     """NMF on a sparse target, beta 1 or 2 (reference: nmf.py:603-638): V is a coalesced sparse COO tensor (N,C) on the device;
     its CSR and CSC forms are built here with torch (data-format plumbing) and the update terms are evaluated at the non-zeros
     only by the library (include/nmf_b200.h: nmfb200_nmf_set_target_sparse)."""
-    kind = "nmf"
 
     def __init__(self, V, W, H, precision="auto"):
         super().__init__()
@@ -319,7 +324,7 @@ class CudaSparseNmfEngine(_CudaEngine):
         self._vmin = float(vals.min()) if nnz else 0.0
         self._vmax = float(vals.max()) if nnz else 0.0
         self._has_zeros = nnz < N * C
-        dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
+        dev_index = self._dev_index
         self._acquire(("nmf", dev_index, N, C, R, "f32"),
                       lambda ref: self._lib.nmfb200_nmf_create(ref, dev_index, N, C, R, _capi.PRECISIONS["f32"]))
         self._loss = torch.zeros(1, dtype=torch.float64, device=self.device)
@@ -340,23 +345,6 @@ class CudaSparseNmfEngine(_CudaEngine):
     def sync(self):
         pass
 
-    def update_w(self, beta, gamma, l1_reg, l2_reg):
-        _capi.check(self._lib.nmfb200_nmf_update_w(self._ctx, _ptr(self.W), _ptr(self.H), beta, gamma, l1_reg,
-                                                   l2_reg, _stream(self.device)))
-
-    def update_h(self, beta, gamma, l1_reg, l2_reg):
-        _capi.check(self._lib.nmfb200_nmf_update_h(self._ctx, _ptr(self.W), _ptr(self.H), beta, gamma, l1_reg,
-                                                   l2_reg, _stream(self.device)))
-
-    def iterate(self, n_iter, beta, gamma, l1_reg, l2_reg):
-        _capi.check(self._lib.nmfb200_nmf_iterate(self._ctx, _ptr(self.W), _ptr(self.H), beta, gamma, l1_reg, l2_reg,
-                                                  int(n_iter), _stream(self.device)))
-
-    def loss_tensor(self, beta):
-        _capi.check(self._lib.nmfb200_nmf_loss(self._ctx, _ptr(self.W), _ptr(self.H), beta, _ptr(self._loss),
-                                               _stream(self.device)))
-        return self._loss
-
 
 class CudaNmfdEngine(_CudaEngine):
     """NMFD / NMF2D / NMF3D on one GPU: V (B,C,*X), W (C,R,*K), H (B,R,*(X-K+1)) over one to three convolved axes."""
@@ -373,7 +361,7 @@ class CudaNmfdEngine(_CudaEngine):
         assert 1 <= nd <= 3 and len(K) == nd
         assert W.shape == (C, R, *K) and H.shape == (B, R, *(x - k + 1 for x, k in zip(X, K)))
         self.V, self.W, self.H = V, W, H
-        dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
+        dev_index = self._dev_index
         if nd == 1:
             create = lambda ref: self._lib.nmfb200_nmfd_create(ref, dev_index, B, C, X[0], R, K[0],
                                                                _capi.PRECISIONS[precision])
@@ -389,30 +377,6 @@ class CudaNmfdEngine(_CudaEngine):
 
     def sync(self):
         _capi.check(self._lib.nmfb200_nmfd_sync_factors(self._ctx))
-
-    def raw_terms(self, which, beta):
-        """(numerator, denominator) of the update of W (which=0) or H (which=1) from the CURRENT factors, untouched, in
-        the factor's own shape; the denominator is (R,) for beta == 1 (include/nmf_b200.h: nmfb200_nmfd_raw_terms)."""
-        f = self.W if which == 0 else self.H
-        n = int(self._lib.nmfb200_nmfd_raw_terms_numel(self._ctx, int(which), float(beta)))
-        buf = torch.empty(n, dtype=torch.float32, device=self.device)
-        _capi.check(self._lib.nmfb200_nmfd_raw_terms(self._ctx, _ptr(self.W), _ptr(self.H), int(which), float(beta),
-                                                     _ptr(buf), _stream(self.device)))
-        num, den = buf[:f.numel()].view(f.shape), buf[f.numel():]
-        return num, (den if beta == 1 else den.view(f.shape))
-
-    def update_w(self, beta, gamma, l1_reg, l2_reg):
-        _capi.check(self._lib.nmfb200_nmfd_update_w(self._ctx, _ptr(self.W), _ptr(self.H), beta, gamma, l1_reg,
-                                                    l2_reg, _stream(self.device)))
-
-    def update_h(self, beta, gamma, l1_reg, l2_reg):
-        _capi.check(self._lib.nmfb200_nmfd_update_h(self._ctx, _ptr(self.W), _ptr(self.H), beta, gamma, l1_reg,
-                                                    l2_reg, _stream(self.device)))
-
-    def loss_tensor(self, beta):
-        _capi.check(self._lib.nmfb200_nmfd_loss(self._ctx, _ptr(self.W), _ptr(self.H), beta, _ptr(self._loss),
-                                                _stream(self.device)))
-        return self._loss
 
 
 class ShardedEngine:
